@@ -3,6 +3,10 @@
 
     python bench.py --gpus N --steps K --warmup W          # our arm (CUDA, one rank per GPU)
     python bench.py --impl reference --gpus N ...          # reference CPU path on the host cores
+    python bench.py ... --dump-outputs DIR                 # also save the last timed step's kNN indices
+
+--steps is the number of timed steps in either arm.  The inputs are seeded, so two builds run with the same
+arguments can be compared output for output through --dump-outputs.
 
 A "step" is one pass of the fused pairwise-distance + kNN kernel over one batch of BASELINE
 config C2 (B=32 clouds of N=1024 points, k=20 — the DGCNN graph).  Weak scaling: every rank owns
@@ -31,7 +35,8 @@ FLOP_PER_PAIR = 8
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=2000)
+    ap.add_argument("--steps", type=int, default=2000,
+                    help="timed steps (the reference arm runs on the host at ~0.1-0.2 s per step: pass a few dozen)")
     ap.add_argument("--warmup", type=int, default=20)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true", help="skip the ~10 s oracle timing")
@@ -39,7 +44,21 @@ def parse():
     ap.add_argument("--no-graph", action="store_true", help="launch every step directly (no CUDA graph)")
     ap.add_argument("--profile", action="store_true",
                     help="for runs under ncu: no clock ramp, no CPU baseline, few secondary iterations")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the kNN indices of the last timed step to DIR/knn_idx.npy (float64)")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    return args
+
+
+def dump_outputs(directory, **arrays):
+    """Save each array as DIR/<name>.npy in float64, so that two builds run with the same arguments (hence the
+    same seeded inputs) can be compared output for output."""
+    import numpy as np
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), np.asarray(a, dtype=np.float64))
 
 
 def peaks():
@@ -140,13 +159,15 @@ def run_reference(args, rank):
         if best_t is None or dt < best_t:
             best_t, cores = dt, c
     torch.set_num_threads(cores)
-    steps = max(1, min(args.steps, 200))
-    for _ in range(max(1, min(args.warmup, 3))):
+    steps = args.steps
+    for _ in range(args.warmup):
         ref_torch.knn(x, K_NN)
     t0 = time.perf_counter()
     for _ in range(steps):
-        ref_torch.knn(x, K_NN)
+        idx = ref_torch.knn(x, K_NN)
     el = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, knn_idx=idx.numpy())
     value = steps * B_PER_GPU * N_PTS * N_PTS / el
     sample = "torch-CPU knn() restatement, %d steps of one B=%d N=%d k=%d batch, %d threads" % (
         steps, B_PER_GPU, N_PTS, K_NN, cores)
@@ -241,6 +262,8 @@ def run_ours(args, rank, local_rank, world):
     # kernels of ours executed in the timed region: graph nodes replayed + direct launches
     launches = replays * per_replay + (_C.launch_count() - l0)
     ms = e0.elapsed_time(e1)
+    # the buffer the last timed step wrote: the last direct launch, else the last node of the graph
+    last_idx = outs[(direct - 1) % pool if direct else per_replay - 1].cpu() if args.dump_outputs else None
     if dist_on:
         t = torch.tensor([ms], device=dev)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -329,6 +352,8 @@ def run_ours(args, rank, local_rank, world):
             line["extra"] = extra
         if world == 1 and not args.no_cpu_baseline and not args.profile:
             line["cpu_baseline"] = cpu_baseline_port(args.cpu_seconds)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, knn_idx=last_idx.numpy())
         print(json.dumps(line), flush=True)
     if dist_on:
         dist.destroy_process_group()

@@ -220,12 +220,90 @@ def gen_rpm():
          a2=a2.numpy(), b2=b2.numpy(), w2=w2.numpy(), T2=T2.numpy())
 
 
+def live_inputs(kind, seed):
+    """Seeded inputs of tests/test_oracle_vs_live_reference.py (the test draws them again)."""
+    if kind == "knn":
+        rng = np.random.default_rng(500 + seed)
+        B, N, k = int(rng.integers(1, 4)), int(rng.integers(40, 400)), int(rng.integers(1, 30))
+        return rng.random((B, 3, N), dtype=np.float32), k
+    rng = np.random.default_rng((700 if kind == "group" else 900) + seed)
+    B, N, S = 2, int(rng.integers(50, 300) if kind == "group" else rng.integers(64, 200)), int(
+        rng.integers(5, 40) if kind == "group" else rng.integers(8, 32))
+    xyz = rng.random((B, N, 3), dtype=np.float32)
+    return xyz, np.ascontiguousarray(xyz[:, :S]), rng
+
+
+def gen_live():
+    """The reference's pure-torch kNN / grouping helpers (utils/model_common_utils.py, pointconv_util.py,
+    ppfnet_util.py) on the seeded inputs of live_inputs(); large outputs as a seeded sample."""
+    from learning3d.utils import model_common_utils as mcu
+    from learning3d.utils import pointconv_util as pcu
+    from learning3d.utils import ppfnet_util as ppf
+    out = {}
+    for seed in range(4):
+        x, k = live_inputs("knn", seed)
+        xt = torch.from_numpy(x)
+        feat = mcu.get_graph_feature(xt, k=k, device="cpu").numpy()
+        flat = np.sort(np.random.default_rng(seed).choice(feat.size, 512, replace=False))
+        rows = np.sort(np.random.default_rng(seed).choice(x.shape[2], min(x.shape[2], 96), replace=False))
+        out["knn%d_rows" % seed] = rows.astype(np.int16)
+        out["knn%d_idx" % seed] = mcu.knn(xt, k).numpy()[:, rows].astype(np.int16)
+        out["knn%d_feat_flat" % seed], out["knn%d_feat" % seed] = flat.astype(np.int32), feat.reshape(-1)[flat]
+    for seed in range(3):
+        xyz, new_xyz, rng = live_inputs("group", seed)
+        t_xyz, t_new = torch.from_numpy(xyz), torch.from_numpy(new_xyz)
+        sd = mcu.square_distance(t_new, t_xyz).numpy()
+        flat = np.sort(np.random.default_rng(seed).choice(sd.size, 512, replace=False))
+        out["group%d_sqdist_flat" % seed], out["group%d_sqdist" % seed] = flat.astype(np.int32), sd.reshape(-1)[flat]
+        ns = int(rng.integers(2, 20))
+        idx, cnt = mcu.query_ball_point(0.25, ns, t_xyz, t_new, get_cnt=True)
+        out["group%d_ball_idx" % seed], out["group%d_ball_cnt" % seed] = idx.numpy().astype(np.int16), cnt.numpy()
+        out["group%d_fps" % seed] = mcu.farthest_point_sample(t_xyz, new_xyz.shape[1], start_with_first_point=True).numpy()
+        val, kidx = mcu.knn_point(int(rng.integers(1, 12)), t_xyz, t_new)
+        out["group%d_knn_val" % seed], out["group%d_knn_idx" % seed] = val.numpy(), kidx.numpy().astype(np.int16)
+    for seed in range(2):
+        xyz, new_xyz, rng = live_inputs("pointconv", seed)
+        t_xyz, t_new = torch.from_numpy(xyz), torch.from_numpy(new_xyz)
+        S = new_xyz.shape[1]
+        out["pc%d_knn" % seed] = pcu.knn_point(int(rng.integers(2, 16)), t_xyz, t_new).numpy().astype(np.int16)
+        out["pc%d_fps" % seed] = pcu.farthest_point_sample(t_xyz, S).numpy()
+        out["pc%d_density" % seed] = pcu.compute_density(t_xyz, 0.2).numpy()
+        itself = torch.arange(S).view(1, S).repeat(2, 1)
+        out["pc%d_ppf_ball" % seed] = ppf.query_ball_point(0.3, 12, t_xyz, t_new, itself).numpy().astype(np.int16)
+    save("live_reference", **out)
+
+
+def gen_compiled_chamfer():
+    """The reference's Chamfer extension (cd.forward = nnsearch on CPU) on a ragged pair of clouds."""
+    import learning3d.losses.cuda.chamfer_distance as ref_cd_pkg   # JIT-builds `cd`
+    rng = np.random.default_rng(7)
+    a, b = torch.from_numpy(rng.random((2, 257, 3), dtype=np.float32)), torch.from_numpy(rng.random((2, 130, 3), dtype=np.float32))
+    d1, d2 = torch.zeros(2, 257), torch.zeros(2, 130)
+    i1, i2 = torch.zeros(2, 257, dtype=torch.int), torch.zeros(2, 130, dtype=torch.int)
+    ref_cd_pkg.chamfer_distance.cd.forward(a, b, d1, d2, i1, i2)
+    save("chamfer_compiled", dist1=d1.numpy(), dist2=d2.numpy(), idx1=i1.numpy(), idx2=i2.numpy())
+
+
+def gen_checkpoints():
+    """Parameter names and shapes of the reference's pretrained FlowNet3D and DCP checkpoints (the weights
+    themselves are too large to keep): the models' state_dict layout must stay loadable."""
+    import json
+    out = {}
+    for ck in ("exp_flownet/models/model.best.t7", "exp_dcp/models/best_model.t7"):
+        sd = torch.load(os.path.join(REF, "pretrained", ck), map_location="cpu", weights_only=False)
+        out[ck] = {k: list(v.shape) for k, v in sd.items()}
+    path = os.path.join(HERE, "reference_checkpoints.json")
+    with open(path, "w") as f:
+        json.dump(out, f, indent=0, sort_keys=True)
+    print("wrote", path)
+
+
 if __name__ == "__main__":
     os.environ.setdefault("TORCH_CUDA_ARCH_LIST", "10.0")
     os.environ.setdefault("TORCH_EXTENSIONS_DIR", tempfile.mkdtemp(prefix="l3dref_ext_"))
     os.environ["CC"] = "/usr/bin/gcc"; os.environ["CXX"] = "/usr/bin/g++"
     import_reference()
-    which = sys.argv[1:] or ["knn", "chamfer", "group", "svd", "dcp", "rpm"]
+    which = sys.argv[1:] or ["knn", "chamfer", "group", "svd", "dcp", "rpm", "live", "chamfer_compiled", "checkpoints"]
     if "rpm" in which:
         gen_rpm()
     if "knn" in which:
@@ -238,3 +316,9 @@ if __name__ == "__main__":
         gen_svd()
     if "dcp" in which:
         gen_dcp()
+    if "live" in which:
+        gen_live()
+    if "chamfer_compiled" in which:
+        gen_compiled_chamfer()
+    if "checkpoints" in which:
+        gen_checkpoints()

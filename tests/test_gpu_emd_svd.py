@@ -180,41 +180,35 @@ def test_svd_head_module_is_trainable(golden_dir):
 
 
 @pytest.mark.parametrize("B,n,m", [(8, 1024, 1024), (2, 300, 700)])
-def test_emd_against_reference_cuda_kernels(B, n, m):
-    """The reference's OWN approxmatch / matchcost / matchcostgrad kernels (emd.cuh compiled in place into
-    oracle/_ref/libemd_ref.so) run on this GPU: pins the EMD path against a running reference.
-    cost 1e-5 relative; row/column masses 2e-5; single match entries within the soft-assignment jitter."""
-    import ctypes
-    ref = oe.ref_emd()
-    if ref is None:
-        pytest.skip("oracle/_ref/libemd_ref.so not present")
+def test_emd_against_reference_cuda_kernels(B, n, m, golden_dir):
+    """The reference's OWN approxmatch / matchcost / matchcostgrad kernels (emd.cuh), recorded on a B200 by
+    tests/golden/make_golden_gpu.py (seeded samples of the large outputs): pins the EMD path against the
+    reference.  cost 1e-5 relative; row/column masses 2e-5; single match entries within the soft-assignment jitter."""
     from learning3d_b200 import _C
+    from oracle import seeded
+    g = np.load(f"{golden_dir}/ref_gpu.npz")
+    tag = "emd_%d_%d_%d_" % (B, n, m)
+    cols, rows = seeded.sample_index(n, 64, tag + "cols"), seeded.sample_index(m, 64, tag + "rows")
     lib = _C.lib()
     rng = np.random.default_rng(B + n)
     a = T(rng.random((B, n, 3), dtype=np.float32)); b = T(rng.random((B, m, 3), dtype=np.float32))
-    P = lambda t: ctypes.c_void_p(t.data_ptr())
-    rmatch = torch.zeros((B, n, m), device=DEV); rtemp = torch.zeros((B, 2 * (n + m)), device=DEV)
-    rcost = torch.zeros((B,), device=DEV)
-    ref.ref_emd_forward(B, n, m, P(a), P(b), P(rmatch), P(rtemp), P(rcost))
-    torch.cuda.synchronize()
     cost = torch.empty((B,), device=DEV); match = torch.empty((B, n, m), device=DEV)
     ws = torch.empty(int(lib.l3d_emd_forward_ws_bytes(B, n, m)), dtype=torch.uint8, device=DEV)
     _C.check(lib.l3d_emd_forward(_C.ptr(a), _C.ptr(b), B, n, m, _C.ptr(cost), _C.ptr(match), _C.ptr(ws), _C.stream()))
     torch.cuda.synchronize()
-    np.testing.assert_allclose(cost.cpu().numpy(), rcost.cpu().numpy(), rtol=1e-5)
-    mm, rm = match.cpu().numpy().reshape(B, m, n), rmatch.cpu().numpy().reshape(B, m, n)
-    np.testing.assert_allclose(mm.sum(1), rm.sum(1), atol=2e-5)
-    np.testing.assert_allclose(mm.sum(2), rm.sum(2), atol=1e-3)
-    np.testing.assert_allclose(mm, rm, atol=5e-3)
-    # gradients on the reference's own matching
-    rg1 = torch.zeros_like(a); rg2 = torch.zeros_like(b)
-    ref.ref_emd_backward(B, n, m, P(a), P(b), P(rmatch), P(rg1), P(rg2))
+    np.testing.assert_allclose(cost.cpu().numpy(), g[tag + "cost"], rtol=1e-5)
+    mm = match.cpu().numpy().reshape(B, m, n)
+    np.testing.assert_allclose(mm.sum(1)[:, cols], g[tag + "colsum"], atol=2e-5)
+    np.testing.assert_allclose(mm.sum(2)[:, rows], g[tag + "rowsum"], atol=1e-3)
+    np.testing.assert_allclose(mm.reshape(-1)[seeded.sample_index(mm.size, 1024, tag + "flat")], g[tag + "entries"], atol=5e-3)
+    # gradients on the same fixed matching the reference's backward was given
+    fixed = T(np.random.default_rng(B + n + 1).random((B, m, n), dtype=np.float32) * np.float32(2.0 / (n + m)))
     g1 = torch.empty_like(a); g2 = torch.empty_like(b)
     ws2 = torch.empty(int(lib.l3d_emd_backward_ws_bytes(B, n, m)), dtype=torch.uint8, device=DEV)
-    _C.check(lib.l3d_emd_backward(_C.ptr(a), _C.ptr(b), _C.ptr(rmatch), B, n, m, _C.ptr(g1), _C.ptr(g2), _C.ptr(ws2), _C.stream()))
+    _C.check(lib.l3d_emd_backward(_C.ptr(a), _C.ptr(b), _C.ptr(fixed), B, n, m, _C.ptr(g1), _C.ptr(g2), _C.ptr(ws2), _C.stream()))
     torch.cuda.synchronize()
-    np.testing.assert_allclose(g1.cpu().numpy(), rg1.cpu().numpy(), rtol=1e-4, atol=1e-5)
-    np.testing.assert_allclose(g2.cpu().numpy(), rg2.cpu().numpy(), rtol=1e-4, atol=1e-5)
+    np.testing.assert_allclose(g1.cpu().numpy()[:, cols], g[tag + "grad1"], rtol=1e-4, atol=1e-5)
+    np.testing.assert_allclose(g2.cpu().numpy()[:, rows], g[tag + "grad2"], rtol=1e-4, atol=1e-5)
 
 
 @pytest.mark.parametrize("B,n,m", [(8, 1024, 1024), (3, 300, 700), (20, 512, 256), (1, 50, 33)])

@@ -1,8 +1,6 @@
 """GPU parity: grouping family through the C ABI / the drop-in Python modules, against the oracle, the
-reference-generated fixtures and (when oracle/_ref/libpn2_ref.so travelled) the reference's own
-pointnet2 CUDA kernels run on the same GPU."""
-import ctypes
-
+reference-generated fixtures (the oracle itself is pinned to the reference's own pointnet2 CUDA kernels by
+tests/test_oracle_group.py::test_reference_cuda_kernels_agree_with_oracle)."""
 import numpy as np
 import pytest
 import torch
@@ -20,15 +18,6 @@ def T(a):
 @pytest.fixture(scope="module")
 def g(golden_dir):
     return np.load(f"{golden_dir}/group.npz")
-
-
-@pytest.fixture(scope="module")
-def ref():
-    return og.ref_pn2()
-
-
-def _p(t):
-    return ctypes.c_void_p(t.data_ptr())
 
 
 # ---- torch-semantics helpers vs the real reference's outputs ---------------------------------
@@ -179,55 +168,3 @@ def test_query_and_group_module():
     want = np.concatenate([gx, og.pn2_group_points(feats, idx)], 1)
     assert out.shape == (2, 12, 64, 16) and np.array_equal(out.cpu().numpy(), want)
     assert pu.GroupAll()(T(xyz), None, T(feats)).shape == (2, 12, 1, 400)
-
-
-# ---- the reference's own CUDA kernels on this GPU pin the oracle ------------------------------------
-def test_reference_cuda_kernels_agree_with_oracle(ref, oracle_mod):
-    if ref is None:
-        pytest.skip("oracle/_ref/libpn2_ref.so not present")
-    rng = np.random.default_rng(12)
-    B, N, S = 4, 2048, 512
-    xyz = (rng.random((B, N, 3), dtype=np.float32) * 2 - 1).astype(np.float32)
-    new_xyz = np.ascontiguousarray(xyz[:, :S])
-    xd, qd = T(xyz), T(new_xyz)
-    s = ctypes.c_void_p(torch.cuda.current_stream().cuda_stream)
-    # ball query (K7)
-    idx = torch.zeros((B, S, 16), dtype=torch.int32, device=DEV)
-    ref.ref_ball_query(B, N, S, ctypes.c_float(0.2), 16, _p(qd), _p(xd), _p(idx), s)
-    torch.cuda.synchronize()
-    assert np.array_equal(idx.cpu().numpy(), og.pn2_ball_query(0.2, 16, xyz, new_xyz))
-    # kNN (K11) and three_nn (K12)
-    for k in (8, 64):
-        d2 = torch.empty((B, S, k), device=DEV); ik = torch.empty((B, S, k), dtype=torch.int32, device=DEV)
-        ref.ref_knn(B, S, N, k, _p(qd), _p(xd), _p(d2), _p(ik), s)
-        torch.cuda.synchronize()
-        od2, oi = oracle_mod.pn2_knn(k, new_xyz, xyz)
-        assert np.array_equal(ik.cpu().numpy(), oi) and np.array_equal(d2.cpu().numpy(), od2)
-    d3 = torch.empty((B, S, 3), device=DEV); i3 = torch.empty((B, S, 3), dtype=torch.int32, device=DEV)
-    ref.ref_three_nn(B, S, N, _p(qd), _p(xd), _p(d3), _p(i3), s)
-    torch.cuda.synchronize()
-    od3, oi3 = oracle_mod.pn2_knn(3, new_xyz, xyz)
-    assert np.array_equal(i3.cpu().numpy(), oi3) and np.array_equal(d3.cpu().numpy(), od3)
-    # FPS (K10), including a duplicated cloud (tie rule of the shared-memory tree)
-    for cloud in (xyz, np.tile(xyz[:, :256], (1, 4, 1))):
-        n = cloud.shape[1]
-        temp = torch.full((B, n), 1e10, device=DEV); fi = torch.empty((B, 300), dtype=torch.int32, device=DEV)
-        cd_ = T(cloud)
-        ref.ref_fps(B, n, 300, _p(cd_), _p(temp), _p(fi), s)
-        torch.cuda.synchronize()
-        want, wtemp = og.pn2_fps(cloud, 300)
-        assert np.array_equal(fi.cpu().numpy(), want)
-        assert np.array_equal(temp.cpu().numpy(), wtemp)
-    # group / interpolate
-    feats = rng.standard_normal((B, 10, N)).astype(np.float32)
-    gi = rng.integers(0, N, (B, 64, 8)).astype(np.int32)
-    out = torch.empty((B, 10, 64, 8), device=DEV)
-    fd, gid = T(feats), T(gi)          # keep the device tensors alive across the async launches
-    ref.ref_group_points(B, 10, N, 64, 8, _p(fd), _p(gid), _p(out), s)
-    w = rng.random((B, S, 3)).astype(np.float32); ti = rng.integers(0, N, (B, S, 3)).astype(np.int32)
-    o3 = torch.empty((B, 10, S), device=DEV)
-    tid, wd = T(ti), T(w)
-    ref.ref_three_interpolate(B, 10, N, S, _p(fd), _p(tid), _p(wd), _p(o3), s)
-    torch.cuda.synchronize()
-    assert np.array_equal(out.cpu().numpy(), og.pn2_group_points(feats, gi))
-    assert np.array_equal(o3.cpu().numpy(), og.pn2_three_interpolate(feats, ti, w))

@@ -83,9 +83,27 @@ def test_tail_gradients_take_the_torch_path():
         np.testing.assert_allclose(R.sinkhorn(-d.detach(), 3, True).cpu().numpy(), lp.detach().cpu().numpy(), atol=5e-5)
 
 
-def test_square_distance_dispatch_and_reference_rpmnet_rebound():
-    """learning3d_b200.utils.square_distance accepts C != 3 now; the reference's own rpmnet functions, rebound,
-    return what the unmodified ones return on this GPU."""
+def _check_rpm_tail(R, golden_dir):
+    """RPMNet's matching tail through the rpmnet module `R` against what the reference's own rpmnet functions,
+    unmodified, returned on a B200 (tests/golden/make_golden_gpu.py, seeded samples)."""
+    from oracle import seeded
+    g = np.load(f"{golden_dir}/ref_gpu.npz")
+    with torch.no_grad():
+        d, lp, T = seeded.rpm_tail(R, *[t.to(DEV) for t in seeded.rpm_inputs()])
+    np.testing.assert_allclose(d.cpu().numpy().reshape(-1)[seeded.sample_index(d.numel(), 1024, "rpm_d")], g["rpm_d"], atol=1e-4)
+    np.testing.assert_allclose(lp.cpu().numpy().reshape(-1)[seeded.sample_index(lp.numel(), 1024, "rpm_lp")], g["rpm_lp"], atol=2e-4)
+    np.testing.assert_allclose(T.cpu().numpy(), g["rpm_T"], atol=2e-5)
+
+
+def test_rpmnet_tail_matches_reference_fixture(golden_dir):
+    """Our rpmnet functions (learning3d_b200.models.rpmnet) return what the reference's returned."""
+    from learning3d_b200.models import rpmnet as ours
+    _check_rpm_tail(ours, golden_dir)
+
+
+def test_square_distance_dispatch_and_reference_rpmnet_rebound(golden_dir):
+    """learning3d_b200.utils.square_distance accepts C != 3 now; the reference's own rpmnet functions, rebound to
+    libl3d_b200.so (learning3d_b200.bind), return what the unmodified ones returned."""
     from learning3d_b200.utils import square_distance
     from oracle import ref_pkg
     x = torch.randn(2, 40, 7, device=DEV); y = torch.randn(2, 30, 7, device=DEV)
@@ -94,28 +112,11 @@ def test_square_distance_dispatch_and_reference_rpmnet_rebound():
         pytest.skip("reference package not staged")
     from learning3d_b200 import bind
     ref = ref_pkg.import_reference()
-    Rr = ref.models.rpmnet
-    torch.manual_seed(5)
-    fs = 0.3 * torch.randn(4, 717, 96, device=DEV); fr = 0.3 * torch.randn(4, 717, 96, device=DEV)
-    fr[:, :300] = fs[:, :300] + 0.03 * torch.randn(4, 300, 96, device=DEV)
-    xyz_ref = torch.rand(4, 717, 3, device=DEV) - 0.5; xyz_src = torch.rand(4, 717, 3, device=DEV) - 0.5
-
-    def run():
-        d = Rr.match_features(fs, fr)
-        lp = Rr.sinkhorn(-2.0 * (d - 0.5), n_iters=5, slack=True)
-        perm = torch.exp(lp)
-        wt = perm @ xyz_ref / (torch.sum(perm, dim=2, keepdim=True) + 1e-5)
-        return d, lp, Rr.compute_rigid_transform(xyz_src, wt, weights=torch.sum(perm, dim=2))
-    with torch.no_grad():
-        want = run()
-        bind.bind(ref)
-        try:
-            got = run()
-        finally:
-            bind.unbind(ref)
-    np.testing.assert_allclose(got[0].cpu().numpy(), want[0].cpu().numpy(), atol=1e-4)
-    np.testing.assert_allclose(got[1].cpu().numpy(), want[1].cpu().numpy(), atol=2e-4)
-    np.testing.assert_allclose(got[2].cpu().numpy(), want[2].cpu().numpy(), atol=2e-5)
+    bind.bind(ref)
+    try:
+        _check_rpm_tail(ref.models.rpmnet, golden_dir)
+    finally:
+        bind.unbind(ref)
 
 
 def test_knn_point_on_features():

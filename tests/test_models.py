@@ -1,20 +1,22 @@
-"""Callers of the hot path (API-compat): state_dict compatibility with the reference's checkpoints (CPU, only
-where /root/reference exists) and GPU forward checks."""
-import os
+"""Callers of the hot path (API-compat): state_dict compatibility with the reference's checkpoints (CPU) and GPU
+forward checks."""
+import json
 
 import numpy as np
 import pytest
 import torch
 
-REF = "/root/reference/pretrained"
 
-
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference checkpoints only exist in the build container")
-def test_reference_checkpoints_load():
+def test_reference_checkpoints_load(golden_dir):
+    """The parameter names and shapes of the reference's pretrained FlowNet3D and DCP checkpoints (recorded by
+    tests/golden/make_golden.py gen_checkpoints) load strictly into our modules."""
     from learning3d_b200.models import DGCNN, FlowNet3D
-    sd = torch.load(f"{REF}/exp_flownet/models/model.best.t7", map_location="cpu", weights_only=False)
+    with open(f"{golden_dir}/reference_checkpoints.json") as f:
+        shapes = json.load(f)
+    ckpt = lambda name: {k: torch.zeros(s) for k, s in shapes[name].items()}
+    sd = ckpt("exp_flownet/models/model.best.t7")
     FlowNet3D().load_state_dict(sd, strict=True)                   # identical module tree / names
-    dcp = torch.load(f"{REF}/exp_dcp/models/best_model.t7", map_location="cpu", weights_only=False)
+    dcp = ckpt("exp_dcp/models/best_model.t7")
     emb = {k[len("emb_nn."):]: v for k, v in dcp.items() if k.startswith("emb_nn.")}
     DGCNN(emb_dims=512).load_state_dict(emb, strict=True)
     from learning3d_b200.utils import SVDHead

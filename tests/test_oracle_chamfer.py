@@ -1,5 +1,5 @@
 """CPU: Chamfer restatement in the C oracle against fixtures made by the reference's own
-extension (cd.forward / cd.backward on CPU) and, when built, against oracle/_ref/cd_ref.so."""
+extension (cd.forward / cd.backward on CPU)."""
 import numpy as np
 import pytest
 
@@ -25,19 +25,15 @@ def test_chamfer_loss_and_grads(oracle_mod, golden_dir, tag):
     np.testing.assert_allclose(l2, g["loss_grad2"], rtol=1e-5, atol=1e-9)
 
 
-def test_chamfer_against_compiled_reference(oracle_mod):
-    cd = oracle_mod.ref_cd()
-    if cd is None:
-        pytest.skip("oracle/_ref/cd_ref.so not built (needs /root/reference)")
-    import torch
-    torch.manual_seed(7)
-    a, b = torch.rand(2, 257, 3), torch.rand(2, 130, 3)
-    d1, d2 = torch.zeros(2, 257), torch.zeros(2, 130)
-    i1, i2 = torch.zeros(2, 257, dtype=torch.int), torch.zeros(2, 130, dtype=torch.int)
-    cd.forward(a, b, d1, d2, i1, i2)
-    o = oracle_mod.chamfer_forward(a.numpy(), b.numpy())
-    for x, y in zip((d1, d2, i1, i2), o):
-        assert np.array_equal(x.numpy(), y)
+def test_chamfer_against_compiled_reference(oracle_mod, golden_dir):
+    """The reference's compiled extension (cd.forward, its CPU nnsearch) on a ragged pair, recorded by
+    tests/golden/make_golden.py (gen_compiled_chamfer): bit-exact."""
+    g = np.load(f"{golden_dir}/chamfer_compiled.npz")
+    rng = np.random.default_rng(7)
+    a, b = rng.random((2, 257, 3), dtype=np.float32), rng.random((2, 130, 3), dtype=np.float32)
+    o = oracle_mod.chamfer_forward(a, b)
+    for name, y in zip(("dist1", "dist2", "idx1", "idx2"), o):
+        assert np.array_equal(g[name], y), name
 
 
 def test_identical_clouds_give_nonfinite_grads(oracle_mod):

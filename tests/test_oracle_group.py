@@ -83,3 +83,35 @@ def test_group_gather_interpolate_adjoints(oracle_mod):
     g3 = rng.standard_normal(o3.shape).astype(np.float32)
     gp3 = og.pn2_three_interpolate_grad(g3, i3, w, 50)
     assert abs(float((o3.astype(np.float64) * g3).sum()) - float((pts.astype(np.float64) * gp3).sum())) < 1e-3
+
+
+# ---- the reference's own CUDA kernels pin the oracle ---------------------------------------------------
+def test_reference_cuda_kernels_agree_with_oracle(oracle_mod, golden_dir):
+    """Outputs of the reference's pointnet2 kernels on a B200, recorded by tests/golden/make_golden_gpu.py as one
+    SHA-256 digest per cloud (every query row), bit-exact against the oracle."""
+    from oracle import seeded
+    D = seeded.array_digest
+    g = np.load(f"{golden_dir}/ref_gpu.npz")
+    rng = np.random.default_rng(12)
+    B, N, S = 4, 2048, 512
+    xyz = (rng.random((B, N, 3), dtype=np.float32) * 2 - 1).astype(np.float32)
+    new_xyz = np.ascontiguousarray(xyz[:, :S])
+    # ball query (K7)
+    assert np.array_equal(g["pn2_ball"], D(og.pn2_ball_query(0.2, 16, xyz, new_xyz)))
+    # kNN (K11) and three_nn (K12)
+    for k in (8, 64):
+        od2, oi = oracle_mod.pn2_knn(k, new_xyz, xyz)
+        assert np.array_equal(g["pn2_knn%d_idx" % k], D(oi)) and np.array_equal(g["pn2_knn%d_dist2" % k], D(od2))
+    od3, oi3 = oracle_mod.pn2_knn(3, new_xyz, xyz)
+    assert np.array_equal(g["pn2_three_nn_idx"], D(oi3)) and np.array_equal(g["pn2_three_nn_dist2"], D(od3))
+    # FPS (K10), including a duplicated cloud (tie rule of the shared-memory tree)
+    for tag, cloud in (("", xyz), ("_dup", np.tile(xyz[:, :256], (1, 4, 1)))):
+        want, wtemp = og.pn2_fps(cloud, 300)
+        assert np.array_equal(g["pn2_fps%s_idx" % tag], want)
+        assert np.array_equal(g["pn2_fps%s_temp" % tag], D(wtemp))
+    # group / interpolate
+    feats = rng.standard_normal((B, 10, N)).astype(np.float32)
+    gi = rng.integers(0, N, (B, 64, 8)).astype(np.int32)
+    w = rng.random((B, S, 3)).astype(np.float32); ti = rng.integers(0, N, (B, S, 3)).astype(np.int32)
+    assert np.array_equal(g["pn2_group"], D(og.pn2_group_points(feats, gi)))
+    assert np.array_equal(g["pn2_interp"], D(og.pn2_three_interpolate(feats, ti, w)))

@@ -1,26 +1,17 @@
-"""CPU, build container only: the oracle against the UNMODIFIED reference imported live from /root/reference
-on fresh seeds (beyond the committed fixtures).  Skipped where the reference checkout is absent (the GPU box);
-nothing GPU-marked reads /root/reference."""
-import importlib.util
-import os
-
+"""CPU: the oracle against what the UNMODIFIED reference's pure-torch helpers (utils/model_common_utils.py,
+pointconv_util.py, ppfnet_util.py) returned on these seeded inputs, beyond the other fixtures.  The reference's
+outputs were recorded by tests/golden/make_golden.py (gen_live) into tests/golden/live_reference.npz; large
+outputs as a seeded sample."""
 import numpy as np
 import pytest
 import torch
 
 from oracle import group as og
 
-REF = "/root/reference"
-pytestmark = pytest.mark.skipif(not os.path.isdir(REF), reason="reference checkout not present")
-
 
 @pytest.fixture(scope="module")
-def ref():
-    """The pure-torch hot-path file of the reference, loaded by path (it imports only torch)."""
-    spec = importlib.util.spec_from_file_location("ref_model_common_utils", os.path.join(REF, "utils", "model_common_utils.py"))
-    mod = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(mod)
-    return mod
+def ref(golden_dir):
+    return np.load(f"{golden_dir}/live_reference.npz")
 
 
 @pytest.mark.parametrize("seed", range(4))
@@ -29,18 +20,19 @@ def test_knn_and_graph_feature_live(oracle_mod, ref, seed):
     B, N, k = int(rng.integers(1, 4)), int(rng.integers(40, 400)), int(rng.integers(1, 30))
     x = rng.random((B, 3, N), dtype=np.float32)
     xt = torch.from_numpy(x)
-    want = ref.knn(xt, k).numpy()
+    rows = ref["knn%d_rows" % seed]
+    want = ref["knn%d_idx" % seed].astype(np.int64)
     got = oracle_mod.knn_expansion(x, k)
     # torch.topk leaves the order of exactly tied keys unspecified: rows must agree unless their keys tie
     xx = (xt ** 2).sum(1, keepdim=True)
-    pd = (-xx - (-2 * torch.matmul(xt.transpose(2, 1).contiguous(), xt)) - xx.transpose(2, 1).contiguous()).numpy()
-    diff = np.argwhere(want != got)
+    pd = (-xx - (-2 * torch.matmul(xt.transpose(2, 1).contiguous(), xt)) - xx.transpose(2, 1).contiguous()).numpy()[:, rows]
+    diff = np.argwhere(want != got[:, rows])
     for b, i, r in diff:
-        assert pd[b, i, want[b, i, r]] == pd[b, i, got[b, i, r]], (b, i, r)
+        assert pd[b, i, want[b, i, r]] == pd[b, i, got[b, rows[i], r]], (b, i, r)
     assert len(diff) <= 0.01 * want.size
     if len(diff) == 0:
-        feat = ref.get_graph_feature(xt, k=k, device="cpu").numpy()
-        assert np.array_equal(oracle_mod.graph_feature(x, got), feat)
+        flat = ref["knn%d_feat_flat" % seed]
+        assert np.array_equal(oracle_mod.graph_feature(x, got).reshape(-1)[flat], ref["knn%d_feat" % seed])
 
 
 @pytest.mark.parametrize("seed", range(3))
@@ -49,49 +41,36 @@ def test_grouping_functions_live(oracle_mod, ref, seed):
     B, N, S = 2, int(rng.integers(50, 300)), int(rng.integers(5, 40))
     xyz = rng.random((B, N, 3), dtype=np.float32)
     new_xyz = np.ascontiguousarray(xyz[:, :S])
-    t_xyz, t_new = torch.from_numpy(xyz), torch.from_numpy(new_xyz)
-    assert np.array_equal(oracle_mod.square_distance(new_xyz, xyz), ref.square_distance(t_new, t_xyz).numpy())
+    flat = ref["group%d_sqdist_flat" % seed]
+    assert np.array_equal(oracle_mod.square_distance(new_xyz, xyz).reshape(-1)[flat], ref["group%d_sqdist" % seed])
     r, ns = 0.25, int(rng.integers(2, 20))
-    idx, cnt = ref.query_ball_point(r, ns, t_xyz, t_new, get_cnt=True)
     oi, oc = og.query_ball_point(r, ns, xyz, new_xyz, want_cnt=True)
-    assert np.array_equal(oi, idx.numpy()) and np.array_equal(oc, cnt.numpy())
-    fps = ref.farthest_point_sample(t_xyz, S, start_with_first_point=True) if "start_with_first_point" in ref.farthest_point_sample.__code__.co_varnames \
-        else None
-    if fps is not None:
-        assert np.array_equal(og.farthest_point_sample(xyz, S), fps.numpy())
+    assert np.array_equal(oi, ref["group%d_ball_idx" % seed]) and np.array_equal(oc, ref["group%d_ball_cnt" % seed])
+    assert np.array_equal(og.farthest_point_sample(xyz, S), ref["group%d_fps" % seed])
     k = int(rng.integers(1, 12))
-    val, kidx = ref.knn_point(k, t_xyz, t_new)
+    val, kidx = ref["group%d_knn_val" % seed], ref["group%d_knn_idx" % seed]
     ov, oi2 = oracle_mod.knn_point(k, xyz, new_xyz)
-    same = oi2 == kidx.numpy()
+    same = oi2 == kidx
     assert same.mean() > 0.99                       # exact distance ties may order differently
-    np.testing.assert_allclose(ov[same], val.numpy()[same], rtol=2e-7, atol=1e-7)
-
-
-def _load(name):
-    spec = importlib.util.spec_from_file_location("ref_" + name, os.path.join(REF, "utils", name + ".py"))
-    mod = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(mod)
-    return mod
+    np.testing.assert_allclose(ov[same], val[same], rtol=2e-7, atol=1e-7)
 
 
 @pytest.mark.parametrize("seed", range(2))
-def test_pointconv_and_ppfnet_variants_live(oracle_mod, seed):
-    pcu, ppf = _load("pointconv_util"), _load("ppfnet_util")
+def test_pointconv_and_ppfnet_variants_live(oracle_mod, ref, seed):
     rng = np.random.default_rng(900 + seed)
     B, N, S = 2, int(rng.integers(64, 200)), int(rng.integers(8, 32))
     xyz = rng.random((B, N, 3), dtype=np.float32)
     new_xyz = np.ascontiguousarray(xyz[:, :S])
-    t_xyz, t_new = torch.from_numpy(xyz), torch.from_numpy(new_xyz)
     # pointconv knn_point: topk(sorted=False) -> compare as sets per row (pointconv_util.py:107-118)
     ns = int(rng.integers(2, 16))
-    want = np.sort(pcu.knn_point(ns, t_xyz, t_new).numpy(), axis=-1)
+    want = np.sort(ref["pc%d_knn" % seed], axis=-1)
     got = np.sort(oracle_mod.knn_sqdist(xyz, new_xyz, ns), axis=-1)
     assert (want == got).mean() > 0.995
     # start-0 FPS (pointconv_util.py:60-83) and density (:199-209)
-    assert np.array_equal(og.farthest_point_sample(xyz, S), pcu.farthest_point_sample(t_xyz, S).numpy())
-    np.testing.assert_allclose(og.compute_density(xyz, 0.2), pcu.compute_density(t_xyz, 0.2).numpy(), rtol=2e-6)
+    assert np.array_equal(og.farthest_point_sample(xyz, S), ref["pc%d_fps" % seed])
+    np.testing.assert_allclose(og.compute_density(xyz, 0.2), ref["pc%d_density" % seed], rtol=2e-6)
     # ppfnet ball query with the query's own index masked out (ppfnet_util.py:96-131)
-    itself = torch.arange(S).view(1, S).repeat(B, 1)
-    want = ppf.query_ball_point(0.3, 12, t_xyz, t_new, itself).numpy()
-    got = og.query_ball_point(0.3, 12, xyz, new_xyz, itself=itself.numpy())
+    itself = np.tile(np.arange(S), (B, 1))
+    want = ref["pc%d_ppf_ball" % seed]
+    got = og.query_ball_point(0.3, 12, xyz, new_xyz, itself=itself)
     assert np.array_equal(want, got)
