@@ -9,7 +9,8 @@ import os
 import torch
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-# L3D_B200_LIB lets profiles/tune_knn.py load experimental builds of the same library
+# L3D_B200_LIB loads another build of the same library instead of the in-tree one, e.g. a parent commit's
+# build for an A/B comparison of bench.py runs
 LIB_PATH = os.environ.get("L3D_B200_LIB") or os.path.join(_HERE, "libl3d_b200.so")
 _lib = None
 

@@ -9,6 +9,8 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include <mutex>
+
 #define L3D_FULL_MASK 0xffffffffu
 
 // ---- error codes shared with include/l3d_b200.h ------------------------------------
@@ -23,6 +25,33 @@
   } while (0)
 
 namespace l3d {
+
+// ---- host launch set-up ----------------------------------------------------------------
+// Number of SMs of device `dev`, cached per host thread (148, a B200's count, if the query fails).
+inline int sm_count(int dev) {
+  static thread_local int c_dev = -1, c_n = 148;
+  if (dev != c_dev) {
+    int n = 0;
+    c_n = (cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev) == cudaSuccess && n > 0) ? n : 148;
+    c_dev = dev;
+  }
+  return c_n;
+}
+
+// Opts kernel Kern in to `bytes` of dynamic shared memory on device `dev`, once per (kernel, device).  The
+// attribute is shared by every host thread, so it is set under a process-wide lock and never lowered: a size
+// per call would let a thread with a smaller problem lower it under a launch that still needs the larger one.
+// Keyed by the kernel itself, not by its type (every kNN kernel is a void(KnnParams)).
+template <auto Kern>
+cudaError_t raise_smem_once(int dev, size_t bytes) {
+  static std::mutex mu;
+  static uint64_t done_mask = 0;   // bit = device ordinal (ordinals >= 64 set the attribute on every call)
+  std::lock_guard<std::mutex> lock(mu);
+  if (dev < 64 && (done_mask >> dev & 1)) return cudaSuccess;
+  const cudaError_t e = cudaFuncSetAttribute(Kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
+  if (e == cudaSuccess && dev < 64) done_mask |= (uint64_t)1 << dev;
+  return e;
+}
 
 __device__ __forceinline__ int lane_id() { return threadIdx.x & 31; }
 __device__ __forceinline__ int warp_id() { return threadIdx.x >> 5; }

@@ -31,7 +31,6 @@
 #include "launch_count.h"
 
 #include <math.h>
-#include <mutex>
 #include <string.h>
 
 namespace l3d {
@@ -410,25 +409,11 @@ edge_gemm_kernel(const EdgeParams p, const __grid_constant__ CUtensorMap tmap_w,
     int it = 0;
     // Tried and rejected (profiles/r02/README.md): prefetching the activation boxes 12 stages beyond the ring into L2
     // (UTMAPF.L2).  The prefetches queue in the same TMA pipe ahead of the ring's own loads and made every layer
-    // slower (layer 2: 108 -> 183 us, p.v: 188 -> 310 us).  -DL3D_EC_PREFETCH=<stages> rebuilds the experiment.
-#ifndef L3D_EC_PREFETCH
-#define L3D_EC_PREFETCH 0
-#endif
-    constexpr int EC_PF = L3D_EC_PREFETCH;                      // pipeline stages (16-channel slabs) of look-ahead
-    auto prefetch_stage = [&](int j) {                          // j = index in this CTA's (tile, k-block) sequence
-      if (EC_PF == 0 || j >= total) return;
-      const int t = j / num_kb, kb = j - t * num_kb;
-      const EdgeUnit pu = edge_unit(p, cluster_id + t * n_clusters, CTAS, crank);
-#pragma unroll
-      for (int q = 0; q < Cfg::BN_LOCAL / 32; ++q)
-        tma_prefetch_3d(&tmap_x, pu.j0 + (int)crank * Cfg::BN_LOCAL + 32 * q, kb * EC_BK, pu.b);
-    };
-    if (EC_PF > 0 && lane == 0)
-      for (int j = STAGES; j < STAGES + EC_PF; ++j) prefetch_stage(j);
+    // slower (layer 2: 108 -> 183 us, p.v: 188 -> 310 us).  The experiment was removed; its code is in git history
+    // before the change that removed it.
     for (int t = 0; t < my_tiles && ok; ++t) {
       const EdgeUnit un = edge_unit(p, cluster_id + t * n_clusters, CTAS, crank);
       for (int kb = 0; kb < num_kb; ++kb, ++it) {
-        if (EC_PF > 0 && lane == 0) prefetch_stage(it + STAGES + EC_PF);
         const int s = it % STAGES;
         const uint32_t n = (uint32_t)(it / STAGES);
         if (!mbar_wait_bounded(&sh->empty[s], (n & 1u) ^ 1u)) { ok = false; break; }
@@ -560,16 +545,6 @@ __global__ void __launch_bounds__(32 * EC_L1P_Q) edge_l1_pool_kernel(const __gri
 
 using namespace l3d;
 
-static int edge_sm_count(int dev) {
-  static thread_local int c_dev = -1, c_n = 148;
-  if (c_dev != dev) {
-    int n = 0;
-    if (cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev) == cudaSuccess && n > 0) c_n = n;
-    c_dev = dev;
-  }
-  return c_n;
-}
-
 extern "C" int l3d_edgeconv_layer1(const float* x_dev, const int64_t* idx_dev, const float* w_host,
                                    const float* scale_host, const float* shift_host, int B, int N, int k, int C1,
                                    float* h1_dev, float* pool_dev, long long pool_bstride, int pool_coff,
@@ -602,17 +577,17 @@ extern "C" int l3d_edgeconv_layer1(const float* x_dev, const int64_t* idx_dev, c
 // relu(scale * (W . X) + shift) for X [B, K, P], W^T [K, M]; optional full output h_out [B, M, P] and optional max
 // over every group of G consecutive positions -> pool_out[b*pool_bstride + (pool_coff + c)*(P/G) + n].
 template <int GT>
-static cudaError_t edge_set_attrs_gt() {
-  cudaError_t e = cudaFuncSetAttribute(edge_gemm_kernel<1, GT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)edge_smem_bytes<1>());
+static cudaError_t edge_set_attrs_gt(int dev) {
+  cudaError_t e = raise_smem_once<edge_gemm_kernel<1, GT>>(dev, edge_smem_bytes<1>());
   if (e != cudaSuccess) return e;
-  return cudaFuncSetAttribute(edge_gemm_kernel<2, GT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)edge_smem_bytes<2>());
+  return raise_smem_once<edge_gemm_kernel<2, GT>>(dev, edge_smem_bytes<2>());
 }
-static cudaError_t edge_set_attrs() {
-  cudaError_t e = edge_set_attrs_gt<1>();
-  if (e == cudaSuccess) e = edge_set_attrs_gt<20>();
-  if (e == cudaSuccess) e = edge_set_attrs_gt<16>();
-  if (e == cudaSuccess) e = edge_set_attrs_gt<8>();
-  if (e == cudaSuccess) e = edge_set_attrs_gt<64>();
+static cudaError_t edge_set_attrs(int dev) {
+  cudaError_t e = edge_set_attrs_gt<1>(dev);
+  if (e == cudaSuccess) e = edge_set_attrs_gt<20>(dev);
+  if (e == cudaSuccess) e = edge_set_attrs_gt<16>(dev);
+  if (e == cudaSuccess) e = edge_set_attrs_gt<8>(dev);
+  if (e == cudaSuccess) e = edge_set_attrs_gt<64>(dev);
   return e;
 }
 
@@ -652,14 +627,8 @@ static int edge_gemm_launch(const float* wt_dev, const float* x_dev, const float
   int dev = 0;
   cudaGetDevice(&dev);
   {
-    static std::mutex mu;
-    static uint64_t done_mask = 0;
-    std::lock_guard<std::mutex> lock(mu);
-    if (dev >= 64 || !(done_mask >> dev & 1)) {
-      cudaError_t e = edge_set_attrs();
-      if (e != cudaSuccess) return (int)e;
-      if (dev < 64) done_mask |= (uint64_t)1 << dev;
-    }
+    const cudaError_t e = edge_set_attrs(dev);
+    if (e != cudaSuccess) return (int)e;
   }
   void* errp = nullptr;
   cudaError_t e = cudaGetSymbolAddress(&errp, g_edgeconv_error);
@@ -697,7 +666,7 @@ static int edge_gemm_launch(const float* wt_dev, const float* x_dev, const float
     }
   }
 
-  const int sms = edge_sm_count(dev);
+  const int sms = sm_count(dev);
   // (the compile-time-G kernels carry no residual / column-divide code)
   const int gt = (pool_out_dev != nullptr && !residual_dev && !col_div_dev && (G == 20 || G == 16 || G == 8 || G == 64)) ? G : 1;
   if (pair) {

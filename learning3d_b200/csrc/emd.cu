@@ -24,7 +24,6 @@
 #include "launch_count.h"
 
 #include <algorithm>
-#include <mutex>
 
 namespace l3d {
 
@@ -755,9 +754,9 @@ extern "C" int l3d_emd_forward(const float* xyz1_dev, const float* xyz2_dev, int
     int dev = 0;
     cudaGetDevice(&dev);
     if (dev != c_dev) {
-      int occ = 0, sms = 0, coop = 0;
+      int occ = 0, coop = 0;
       cudaDeviceGetAttribute(&coop, cudaDevAttrCooperativeLaunch, dev);
-      cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+      const int sms = sm_count(dev);
       if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, emd_persistent_kernel, EMD_THREADS, 0) != cudaSuccess) occ = 0;
       if (occ > 4) occ = 4;                 // 32 warps/SM: while one item's CTAs sit in a barrier the others sweep
       c_cap = coop ? sms * occ : 0;
@@ -833,13 +832,10 @@ extern "C" int l3d_emd_forward(const float* xyz1_dev, const float* xyz2_dev, int
   fp.match = match_dev; fp.partial = partial; fp.cost = cost_dev; fp.ticket = ticket;
   fp.B = B; fp.n = n; fp.m = m;
   {
-    static std::once_flag once[64];
     int dev = 0;
     cudaGetDevice(&dev);
-    if (dev < 64)
-      std::call_once(once[dev], [] { cudaFuncSetAttribute(emd_final_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)EMD_FINAL_SMEM); });
-    else
-      cudaFuncSetAttribute(emd_final_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)EMD_FINAL_SMEM);
+    const cudaError_t e = raise_smem_once<emd_final_kernel>(dev, EMD_FINAL_SMEM);
+    if (e != cudaSuccess) return (int)e;
   }
   emd_final_kernel<<<dim3(gx_final, B), EMD_THREADS, EMD_FINAL_SMEM, s>>>(fp);
   count_launch();

@@ -236,16 +236,12 @@ static int fps_launch(FpsParams p, cudaStream_t s) {
   const int ppt = (p.N + FPS_THREADS - 1) / FPS_THREADS;
   const size_t smem = (size_t)p.N * 3 * sizeof(float);   // <= 96 KB (N <= 8192)
   if (smem > 40 * 1024) {   // (static shared memory also counts against the 48 KB default)
-    // opt in to > 48 KB of dynamic shared memory (per device; only the two widest instantiations need it)
-    static thread_local int attr_dev = -1;
+    // opt in to > 48 KB of dynamic shared memory (only the two widest instantiations need it)
     int dev = 0;
     cudaGetDevice(&dev);
-    if (attr_dev != dev) {
-      cudaError_t e = cudaFuncSetAttribute(fps_kernel<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024);
-      if (e == cudaSuccess) e = cudaFuncSetAttribute(fps_kernel<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024);
-      if (e != cudaSuccess) return (int)e;
-      attr_dev = dev;
-    }
+    cudaError_t e = raise_smem_once<fps_kernel<8>>(dev, 96 * 1024);
+    if (e == cudaSuccess) e = raise_smem_once<fps_kernel<16>>(dev, 96 * 1024);
+    if (e != cudaSuccess) return (int)e;
   }
   if (ppt <= 1) fps_kernel<1><<<p.B, FPS_THREADS, smem, s>>>(p);
   else if (ppt <= 2) fps_kernel<2><<<p.B, FPS_THREADS, smem, s>>>(p);

@@ -475,15 +475,10 @@ extern "C" int l3d_compute_density(const float* xyz_dev, int B, int N, float two
   if (N <= DENS_MAX_N && B <= 65535 && two_bw2 > 0.f && norm != 0.f) {
     const size_t smem = (size_t)N * sizeof(float4);
     if (smem > 40 * 1024) {
-      static thread_local int attr_dev = -1;
       int dev = 0;
       cudaGetDevice(&dev);
-      if (attr_dev != dev) {
-        cudaError_t e = cudaFuncSetAttribute(density_staged_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                             (int)(DENS_MAX_N * sizeof(float4)));
-        if (e != cudaSuccess) return (int)e;
-        attr_dev = dev;
-      }
+      const cudaError_t e = raise_smem_once<density_staged_kernel>(dev, DENS_MAX_N * sizeof(float4));
+      if (e != cudaSuccess) return (int)e;
     }
     const float c_log2 = (float)(-1.4426950408889634 / (double)two_bw2);
     const float inv_norm_n = (float)(1.0 / ((double)norm * (double)N));

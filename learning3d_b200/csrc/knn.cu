@@ -27,61 +27,35 @@
 #include "launch_count.h"
 
 #include <math.h>
-#include <mutex>
 
 namespace l3d {
 
 
-#ifndef L3D_KNN_THREADS
-#define L3D_KNN_THREADS 256  // 128 (4 CTAs/SM) and 512 measured in profiles/r01 (tune_knn.py)
-#endif
-constexpr int KNN_THREADS = L3D_KNN_THREADS;
+constexpr int KNN_THREADS = 256;  // 128 (4 CTAs/SM) and 512 were slower (profiles/r01)
 constexpr int KNN_WARPS = KNN_THREADS / 32;
 constexpr int KNN_CHUNK = 1024;  // points per bulk-copy staging chunk
-#ifndef L3D_KNN_R
-#define L3D_KNN_R 2
-#endif
-#ifndef L3D_KNN_PDL
-#define L3D_KNN_PDL 1        // programmatic dependent launch between consecutive kNN launches
-#endif
-#ifndef L3D_KNN_ALIGN_GRID
-#define L3D_KNN_ALIGN_GRID 0 // grid = multiple of B (no CTA stages two clouds): measured 34.7 vs 33.4 us, off
-#endif
-#ifndef L3D_KNN_DEFER_QW
-#define L3D_KNN_DEFER_QW 1   // keep "- |q|^2" out of the register keys of the expansion mode (knn_rows_v2)
-#endif
 // Selection variants that were measured and dropped (profiles/r01, DESIGN.md §7): rank-by-counting
 // against the shared-memory survivor list (40.9 us), an FMNMX key/value network with tie fallback
 // (37.2 us) — both slower than the 64-bit composite network below (36.1 us at C2).
-// Register budget: left to ptxas' own heuristic by default (127 registers at R = 2, 2 CTAs/SM), which
-// measured fastest; forcing min-blocks 1..5 (48..167 registers) was 10-35 % slower (profiles/r01).
-#ifdef L3D_KNN_MIN_BLOCKS
-#define L3D_KNN_BOUNDS __launch_bounds__(KNN_THREADS, L3D_KNN_MIN_BLOCKS)
-#else
-#define L3D_KNN_BOUNDS __launch_bounds__(KNN_THREADS)
-#endif
-#ifndef L3D_KNN_TPR_MIN_UNITS
-#define L3D_KNN_TPR_MIN_UNITS 512   // 32-row units below which knn() stays on the warp-per-row-pair kernel (measured tie at 512: profiles/r02/knn_paths_time.txt)
-#endif
+// Register budget: left to ptxas' own heuristic (127 registers at R = 2, 2 CTAs/SM), which measured
+// fastest; forcing min-blocks 1..5 (48..167 registers) was 10-35 % slower (profiles/r01).
+// Also measured and removed (the code is in git history before the change that removed it): a grid
+// rounded to a multiple of B so that no CTA stages two clouds (34.7 vs 33.4 us), and a two-pass
+// packed path that re-evaluates the keys for the survivor mask instead of holding 32 per row in
+// registers (36.9 to 41.0 us against 34.9 us).
+// 32-row units below which knn() stays on the warp-per-row-pair kernel (measured tie at 512:
+// profiles/r02/knn_paths_time.txt)
+constexpr int KNN_TPR_MIN_UNITS = 512;
 constexpr int TPR_K_MAX = 24;
-constexpr int KNN_R = L3D_KNN_R;  // query rows per warp on the k <= 24 path (tuned in profiles/r01)
+constexpr int KNN_R = 2;  // query rows per warp on the k <= 24 path (tuned in profiles/r01)
 constexpr int KNN_SORT_MAX_N = 256;  // clouds this small may be sorted whole (8 keys per lane)
 
-
-#ifndef L3D_KNN_TWO_PASS
-#define L3D_KNN_TWO_PASS 0   // packed path: recompute the keys for the mask instead of holding 32 per row in registers
-#endif
-#ifndef L3D_KNN_TP_UNROLL
-#define L3D_KNN_TP_UNROLL 4  // two-pass path: candidate pairs in flight per loop trip (bounds the live LDS results)
-#endif
-#ifndef L3D_KNN_F32X2
-#define L3D_KNN_F32X2 1      // expansion-mode k <= 24 path: evaluate two candidates per FFMA2 (pair layout below)
-#endif
-// Pair layout of a candidate tile for the packed path: lane l's candidates e and e+1 (e even) of tile t, i.e.
-// points j = t*1024 + e*32 + l and j + 32, sit side by side so that one LDS.128 feeds two FFMA2 operands:
+// Pair layout of a candidate tile for the packed path (expansion-mode k <= 24: two candidates per FFMA2):
+// lane l's candidates e and e+1 (e even) of tile t, i.e. points j = t*1024 + e*32 + l and j + 32, sit side
+// by side so that one LDS.128 feeds two FFMA2 operands:
 //   pair_xy[t*512 + (e/2)*32 + l] = (x_e, x_e+1, y_e, y_e+1),  pair_zw[..] = (z_e, z_e+1, -|c_e|^2, -|c_e+1|^2)
 template <int MODE, int KS>
-struct KnnPairs { static constexpr bool value = (L3D_KNN_F32X2 != 0) && (L3D_KNN_DEFER_QW != 0) && MODE == MODE_EXPANSION_NEG && KS == 1; };
+struct KnnPairs { static constexpr bool value = MODE == MODE_EXPANSION_NEG && KS == 1; };
 
 
 template <int S>
@@ -249,9 +223,7 @@ __device__ __forceinline__ void knn_rows_v2(const KnnParams& p, const float4* __
     // is monotone, the registers only feed the threshold and the survivor mask (survivors are
     // re-evaluated with the full formula below), so the selection stays exact as long as the s-space
     // threshold is lowered to cover every s that can round to the k-th key (thr computation below).
-    constexpr bool DEFER = (L3D_KNN_DEFER_QW != 0) && MODE == MODE_EXPANSION_NEG;
-    constexpr bool TWO_PASS = PAIRS && (L3D_KNN_TWO_PASS != 0);
-    constexpr int TPU = L3D_KNN_TP_UNROLL;
+    constexpr bool DEFER = MODE == MODE_EXPANSION_NEG;
     uint32_t mask[R];
     int cnt[R], incl[R], total[R];
     // the s-space threshold of a row from its sorted lane maxima (mx: lane l holds the l-th largest maximum)
@@ -269,55 +241,6 @@ __device__ __forceinline__ void knn_rows_v2(const KnnParams& p, const float4* __
       }
       return thr;
     };
-    if constexpr (TWO_PASS) {
-      // The 32 keys of a lane are never held in registers: pass 1 keeps only the running lane maximum, pass 2
-      // re-evaluates the same packed expressions (same bits) and turns each key straight into its mask bit.
-      // ~64 registers less per thread (more resident warps) for 64 more FFMA2 per row.
-      const ulonglong2* pxy = pair_xy + t * (KNN_TILE / 2) + lane;
-      const ulonglong2* pzw = pair_zw + t * (KNN_TILE / 2) + lane;
-      unsigned long long qx2[R], qy2[R], qz2[R];
-      float m[R];
-#pragma unroll
-      for (int r = 0; r < R; ++r) {
-        qx2[r] = f2_pack(q[r].x, q[r].x); qy2[r] = f2_pack(q[r].y, q[r].y); qz2[r] = f2_pack(q[r].z, q[r].z);
-        m[r] = -INFINITY;
-      }
-      const unsigned long long two2 = f2_pack(2.0f, 2.0f);
-#pragma unroll TPU
-      for (int pe = 0; pe < 16; ++pe) {
-        const ulonglong2 a = pxy[pe * 32], bz = pzw[pe * 32];
-#pragma unroll
-        for (int r = 0; r < R; ++r) {
-          const unsigned long long dot = f2_fma(qz2[r], bz.x, f2_fma(qy2[r], a.y, f2_mul(qx2[r], a.x)));
-          float s0, s1;
-          f2_unpack(f2_fma(two2, dot, bz.y), s0, s1);
-          m[r] = fmaxf(m[r], fmaxf(s0, s1));
-        }
-      }
-      warp_sort32_keys_desc_x<R>(m, lane);
-      unsigned long long nthr[R];
-      uint32_t neg[R];
-#pragma unroll
-      for (int r = 0; r < R; ++r) {
-        const float thr = row_threshold(r, m[r]);
-        nthr[r] = f2_pack(-thr, -thr);
-        neg[r] = 0u;
-      }
-#pragma unroll TPU
-      for (int pe = 15; pe >= 0; --pe) {
-        const ulonglong2 a = pxy[pe * 32], bz = pzw[pe * 32];
-#pragma unroll
-        for (int r = 0; r < R; ++r) {
-          const unsigned long long dot = f2_fma(qz2[r], bz.x, f2_fma(qy2[r], a.y, f2_mul(qx2[r], a.x)));
-          float s0, s1;
-          f2_unpack(f2_add(f2_fma(two2, dot, bz.y), nthr[r]), s0, s1);
-          neg[r] = __funnelshift_l(__float_as_uint(s1), neg[r], 1);
-          neg[r] = __funnelshift_l(__float_as_uint(s0), neg[r], 1);
-        }
-      }
-#pragma unroll
-      for (int r = 0; r < R; ++r) { mask[r] = ~neg[r]; cnt[r] = __popc(mask[r]); }
-    } else {
     float d[R][32];
     if constexpr (PAIRS) {
       // two candidates per instruction: s = fma(2, fma(qz,cz, fma(qy,cy, qx*cx)), -|c|^2), same op order per lane
@@ -381,7 +304,6 @@ __device__ __forceinline__ void knn_rows_v2(const KnnParams& p, const float4* __
       const uint32_t mk = ~neg;
       mask[r] = mk;
       cnt[r] = __popc(mk);
-    }
     }
 #pragma unroll
     for (int r = 0; r < R; ++r) incl[r] = warp_inclusive_scan(cnt[r], lane);
@@ -455,7 +377,7 @@ __host__ __device__ inline size_t knn_smem_bytes(int N, int KS, bool pairs) {
 }
 
 template <int MODE, int KS, bool SELF, bool CAND_BCN, bool FEAT = false, bool PAIRS = false>
-__global__ void L3D_KNN_BOUNDS knn_kernel(const KnnParams p) {
+__global__ void __launch_bounds__(KNN_THREADS) knn_kernel(const KnnParams p) {
   extern __shared__ __align__(128) unsigned char smem[];
   uint64_t* bar = reinterpret_cast<uint64_t*>(smem);
   float* stage = reinterpret_cast<float*>(smem + 16);
@@ -478,12 +400,10 @@ __global__ void L3D_KNN_BOUNDS knn_kernel(const KnnParams p) {
   }
   __syncthreads();
   uint32_t parity = 0;
-#if L3D_KNN_PDL
   // programmatic dependent launch: let the next launch on the stream start filling SMs as our CTAs
   // retire, and do not touch global memory before the previous launch has fully completed
   asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
   asm volatile("griddepcontrol.wait;" ::: "memory");
-#endif
 
   const long rows_total = (long)p.B * M;
   const long r0 = rows_total * blockIdx.x / gridDim.x;
@@ -694,17 +614,6 @@ __global__ void __launch_bounds__(KNN_STREAM_WARPS * 32) knn_stream_kernel(const
 static thread_local int g_force_slow = 0;   // testing hooks are per host thread
 int knn_force_slow_flag() { return g_force_slow; }   // knn_matrix.cu shares the testing hook
 
-static int sm_count() {
-  static int n = 0;
-  if (n == 0) {
-    int dev = 0;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev);
-    if (n <= 0) n = 148;
-  }
-  return n;
-}
-
 template <int MODE, int KS, bool SELF, bool CAND_BCN, bool FEAT = false, bool PAIRS = false>
 static int knn_launch_t(KnnParams p, cudaStream_t stream) {
   if constexpr (!PAIRS && KnnPairs<MODE, KS>::value) {
@@ -712,24 +621,14 @@ static int knn_launch_t(KnnParams p, cudaStream_t stream) {
     if (knn_smem_bytes(p.N, KS, true) <= KNN_SMEM_LIMIT)
       return knn_launch_t<MODE, KS, SELF, CAND_BCN, FEAT, true>(p, stream);
   }
-  auto kern = knn_kernel<MODE, KS, SELF, CAND_BCN, FEAT, PAIRS>;
+  constexpr auto kern = knn_kernel<MODE, KS, SELF, CAND_BCN, FEAT, PAIRS>;
   const size_t smem = knn_smem_bytes(p.N, KS, PAIRS);
   if (smem > KNN_SMEM_LIMIT) return L3D_ERR_UNSUPPORTED;
   int dev = 0;
   cudaGetDevice(&dev);
-  // The opt-in shared-memory limit is a per-(device, function) attribute shared by every host thread: raise it
-  // ONCE to the architectural maximum (never lower it), under a process-wide lock.  A per-call exact size
-  // would let a second thread with a smaller N lower it under a launch that still needs the larger one.
-  {
-    static std::mutex mu;
-    static uint64_t done_mask = 0;        // bit = device ordinal (ordinals >= 64 set the attribute every call)
-    std::lock_guard<std::mutex> lock(mu);
-    if (dev >= 64 || !(done_mask >> dev & 1)) {
-      cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)KNN_SMEM_LIMIT);
-      if (e != cudaSuccess) return (int)e;
-      if (dev < 64) done_mask |= (uint64_t)1 << dev;
-    }
-  }
+  // raised to the architectural maximum, whatever N this call needs
+  const cudaError_t ae = raise_smem_once<kern>(dev, KNN_SMEM_LIMIT);
+  if (ae != cudaSuccess) return (int)ae;
   // the occupancy query is a host-side driver call (~3 us): cache it per (thread, device, smem size)
   static thread_local int c_dev = -1, c_occ = 0;
   static thread_local size_t c_smem = 0;
@@ -743,36 +642,11 @@ static int knn_launch_t(KnnParams p, cudaStream_t stream) {
   if (occ < 1) return L3D_ERR_UNSUPPORTED;
   if (occ > 4) occ = 4;
   const long rows = (long)p.B * p.M;
-  long grid = (long)sm_count() * occ;          // persistent-style: every CTA resident at once
+  long grid = (long)sm_count(dev) * occ;       // persistent-style: every CTA resident at once
   const long max_useful = (rows + KNN_WARPS - 1) / KNN_WARPS;
   if (grid > max_useful) grid = max_useful;
-#if L3D_KNN_ALIGN_GRID
-  // A CTA whose row range crosses a batch item stages two clouds (two prologues on the critical path).
-  // When a multiple of B is within 5 % of the resident grid, use it: ranges then never cross an item.
-  if (grid > p.B) {
-    const long g2 = grid / p.B * p.B;
-    if (g2 * 20 >= grid * 19) grid = g2;
-  }
-#endif
   if (grid < 1) grid = 1;
-#if L3D_KNN_PDL
-  {
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3((unsigned)grid); cfg.blockDim = dim3(KNN_THREADS);
-    cfg.dynamicSmemBytes = smem; cfg.stream = stream;
-    cudaLaunchAttribute at[1];
-    at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    at[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = at; cfg.numAttrs = 1;
-    cudaError_t le = cudaLaunchKernelEx(&cfg, kern, p);
-    if (le != cudaSuccess) return (int)le;
-  }
-#else
-  kern<<<(unsigned)grid, KNN_THREADS, smem, stream>>>(p);
-#endif
-  count_launch();
-  L3D_LAUNCH_CHECK();
-  return L3D_OK;
+  return knn_launch_pdl(kern, grid, KNN_THREADS, smem, stream, p);
 }
 
 extern "C" int l3d_graph_feature(const float* x_dev, const int64_t* idx_dev, int B, int C, int N, int k,
@@ -782,21 +656,14 @@ template <int MODE, bool SELF, bool CAND_BCN>
 static int knn_stream_launch(KnnParams p, cudaStream_t stream) {
   if (p.k > KNN_STREAM_MAX_K) return L3D_ERR_UNSUPPORTED;
   if (p.idx64 == 2 && p.N > 65536) return L3D_ERR_UNSUPPORTED;          // 16-bit wire format of the host path
-  auto kern = knn_stream_kernel<MODE, SELF, CAND_BCN>;
+  constexpr auto kern = knn_stream_kernel<MODE, SELF, CAND_BCN>;
   const size_t smem = knn_stream_smem_bytes(p.k);
   if (smem > 48 * 1024) {
-    // per-(device, function) attribute: raise it once to the largest size this path can ask for, under a lock
-    static std::mutex mu;
-    static uint64_t done_mask = 0;
+    // raised to the largest size this path can ask for
     int dev = 0;
     cudaGetDevice(&dev);
-    std::lock_guard<std::mutex> lock(mu);
-    if (dev >= 64 || !(done_mask >> dev & 1)) {
-      cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                           (int)knn_stream_smem_bytes(KNN_STREAM_MAX_K));
-      if (e != cudaSuccess) return (int)e;
-      if (dev < 64) done_mask |= (uint64_t)1 << dev;
-    }
+    const cudaError_t e = raise_smem_once<kern>(dev, knn_stream_smem_bytes(KNN_STREAM_MAX_K));
+    if (e != cudaSuccess) return (int)e;
   }
   const long row_blocks = ((long)p.M + KNN_STREAM_WARPS - 1) / KNN_STREAM_WARPS;
   const long grid = (long)p.B * row_blocks;
@@ -819,9 +686,6 @@ static int knn_launch(KnnParams p, cudaStream_t stream) {
   // threshold scheme -> every row takes the exact k-round arg-max scan (O(k N) per row, same ordering rule)
   p.force_slow = (g_force_slow || p.k > 128) ? 1 : 0;
   p.use_tma = ((reinterpret_cast<uintptr_t>(p.cand) & 15u) == 0 && (p.N & 3) == 0) ? 1 : 0;
-#ifdef L3D_KNN_FORCE_NO_TMA   // experiment knob (profiles/build_variants.sh): plain-load staging
-  p.use_tma = 0;
-#endif
   // Heavy selections out of a small cloud (FlowNet3D's flow embedding: k = 64 of N = 256) sort the
   // whole row instead of thresholding it.
   if (p.N <= KNN_SORT_MAX_N && p.k * 8 >= p.N) p.full_sort = 1;
@@ -829,7 +693,7 @@ static int knn_launch(KnnParams p, cudaStream_t stream) {
     // knn() on xyz with enough rows to give every SM sub-partition a warp of 32 rows: thread-per-row kernel
     // (knn_tpr.cu, bit-identical results); smaller batches keep the warp-per-row-pair kernel below
     if (!p.full_sort && !(p.k > TPR_K_MAX) && knn_path_flag() != 1 && knn_tpr_eligible(p) &&
-        (knn_path_flag() == 2 || (long)p.B * (p.N / 32) >= L3D_KNN_TPR_MIN_UNITS))
+        (knn_path_flag() == 2 || (long)p.B * (p.N / 32) >= KNN_TPR_MIN_UNITS))
       return knn_tpr_launch(p, stream);
   }
   if (SELF && CAND_BCN && MODE == MODE_EXPANSION_NEG && p.feat_out) {   // fused get_graph_feature variant

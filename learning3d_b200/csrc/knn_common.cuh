@@ -1,6 +1,7 @@
 // Shared pieces of the kNN kernels (knn.cu: warp-per-row-pair selection, knn_tpr.cu: thread-per-row selection).
 #pragma once
 #include "common.cuh"
+#include "launch_count.h"
 
 namespace l3d {
 
@@ -193,6 +194,24 @@ __device__ __forceinline__ void knn_row_v2(const KnnParams& p, const float4* __r
 
   if (overflow) knn_row_slow<MODE>(p, packed, q, row, lane);
   else knn_store_packed(p, row, lane, best);
+}
+
+// Launches a kNN kernel with programmatic dependent launch: the next launch on the stream may start filling SMs as
+// this one's CTAs retire (the kernels run griddepcontrol.wait before they touch global memory).
+inline int knn_launch_pdl(void (*kern)(KnnParams), long grid, int threads, size_t smem, cudaStream_t stream,
+                          const KnnParams& p) {
+  cudaLaunchConfig_t cfg = {};
+  cfg.gridDim = dim3((unsigned)grid); cfg.blockDim = dim3(threads);
+  cfg.dynamicSmemBytes = smem; cfg.stream = stream;
+  cudaLaunchAttribute at[1];
+  at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+  at[0].val.programmaticStreamSerializationAllowed = 1;
+  cfg.attrs = at; cfg.numAttrs = 1;
+  const cudaError_t le = cudaLaunchKernelEx(&cfg, kern, p);
+  if (le != cudaSuccess) return (int)le;
+  count_launch();
+  L3D_LAUNCH_CHECK();
+  return L3D_OK;
 }
 
 // knn_tpr.cu: thread-per-row kernel for knn() on xyz clouds (k <= 24, N % 32 == 0, N <= 2048)

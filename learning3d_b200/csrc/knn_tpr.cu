@@ -28,7 +28,7 @@
 // feeds two rows — the default; see its header below and profiles/micro/pipes.cu for the measurements behind it).
 // The price is parallelism: a row is a thread, so B*N/32 warps exist in total (1024 at C2 = 6.9 per SM) and
 // the kernel is one wave; the launcher therefore only takes this path when there are enough rows
-// (knn.cu: knn_launch, L3D_KNN_TPR_MIN_UNITS), smaller batches stay on the warp-per-row-pair kernel.
+// (knn.cu: knn_launch, KNN_TPR_MIN_UNITS), smaller batches stay on the warp-per-row-pair kernel.
 // C2 (B=32, N=1024, k=20) on a B200: 33.1 us (knn.cu) -> 25.9 us (profiles/r02/knn_paths_time.txt).
 #include "knn_common.cuh"
 #include "reg_sort.cuh"
@@ -36,7 +36,6 @@
 #include "launch_count.h"
 
 #include <math.h>
-#include <mutex>
 
 namespace l3d {
 
@@ -44,48 +43,33 @@ constexpr int TPR_G = 64;       // candidate groups per row (threshold = k-th la
 constexpr int TPR_CAP = 64;     // survivor-list entries per row (uint16 indices)
 __host__ __device__ inline int tpr_slots(int N) { return N <= 1024 ? 2 : 1; }   // clouds resident per CTA round
 constexpr int TPR_MIN_N = 128, TPR_MAX_N = 2048, TPR_MAX_K = 24;
-
-#ifndef L3D_TPR_EXTRACT
-#define L3D_TPR_EXTRACT 1     // 1: three predicated find-lowest-bit steps per mask word + rare loop; 0: plain loop
-#endif
-#ifndef L3D_TPR_FUSE_THR
-#define L3D_TPR_FUSE_THR 1    // 1: pass 2 evaluates s - thr inside the fma chain (no FADD2), threshold lowered by its error bound
-#endif
-#ifndef L3D_TPR_UNROLL_G
-#define L3D_TPR_UNROLL_G 2    // candidate groups per pass-1 loop trip
-#endif
-#ifndef L3D_TPR_STOP
-#define L3D_TPR_STOP 0       // profiling only: 1..4 = stop a unit after staging / pass 1 / threshold / pass 2
-#endif
-
-constexpr int TPR_UNROLL_G = L3D_TPR_UNROLL_G;
-#ifndef L3D_TPR_DUO
-#define L3D_TPR_DUO 1         // 1: clouds with N % 64 == 0 take the two-warps-per-64-rows kernel (knn_duo_kernel)
-#endif
-__host__ __device__ constexpr int tpr_threads(int R) { return R == 2 ? 128 : 256; }
+constexpr int TPR_THREADS = 256;
 
 // shared memory per resident cloud: pair_xy + pair_zw (8 B per candidate each, npad entries) + float4 (x,y,z,|p|^2)
 // padded to whole KNN_TILEs (the warp-cooperative overflow routine of knn_common.cuh reads whole tiles)
 __host__ __device__ inline int tpr_npad(int N) { return (N + 127) & ~127; }
 __host__ __device__ inline int tpr_ntile(int N) { return ((N + KNN_TILE - 1) / KNN_TILE) * KNN_TILE; }
 __host__ __device__ inline size_t tpr_cloud_bytes(int N) { return (size_t)tpr_npad(N) * 16 + (size_t)tpr_ntile(N) * 16; }
-// per-row index lists (+ the entry dead stores land on once a list is full) and group maxima, [R][..][threads]
-__host__ __device__ constexpr size_t tpr_list_bytes(int R) { return (size_t)R * (TPR_CAP + 1) * tpr_threads(R) * 2; }
-__host__ __device__ constexpr size_t tpr_gmax_bytes(int R) { return (size_t)R * TPR_G * tpr_threads(R) * 4; }
-__host__ __device__ inline size_t tpr_smem_bytes(int N, int R) {
-  return tpr_slots(N) * tpr_cloud_bytes(N) + tpr_list_bytes(R) + tpr_gmax_bytes(R) + (size_t)(tpr_threads(R) / 32) * 64 * 8 + 16;
+// per-row index lists (+ the entry dead stores land on once a list is full) and group maxima, [..][threads]
+constexpr size_t TPR_LIST_BYTES = (size_t)(TPR_CAP + 1) * TPR_THREADS * 2;
+constexpr size_t TPR_GMAX_BYTES = (size_t)TPR_G * TPR_THREADS * 4;
+__host__ __device__ inline size_t tpr_smem_bytes(int N) {
+  return tpr_slots(N) * tpr_cloud_bytes(N) + TPR_LIST_BYTES + TPR_GMAX_BYTES + (size_t)(TPR_THREADS / 32) * 64 * 8 + 16;
 }
 
-// R:   query rows per thread (a warp owns 32 R consecutive rows of one cloud).  Shared-memory operand traffic per
-//      row is 1 / R: the micro-benchmark (profiles/micro/pipes.cu) puts a broadcast LDS.128 at 2 SM-cycles per warp
-//      instruction whatever the number of distinct addresses, so at R = 1 the 2 x 1024 operand loads of a row
-//      out-weigh its 2 x 2048 FFMA2 (2 scheduler-cycles each, four schedulers) two to one.
+// One query row per thread, a warp owns 32 consecutive rows of one cloud.  The micro-benchmark
+// (profiles/micro/pipes.cu) puts a broadcast LDS.128 at 2 SM-cycles per warp instruction whatever the number of
+// distinct addresses, so the 2 x 1024 operand loads of a row out-weigh its 2 x 2048 FFMA2 (2 scheduler-cycles each,
+// four schedulers) two to one; knn_duo_kernel below halves them.
 // PPG: candidate pairs per group when known at compile time (8 <=> N = 1024), 0 = run-time.
 // KT:  k when known at compile time (20, DGCNN / DCP), 0 = run-time k <= 24.
-template <int R, int PPG, int KT, bool FEAT>
-__global__ void __launch_bounds__(tpr_threads(R), 1) knn_tpr_kernel(const KnnParams p) {
+template <int PPG, int KT, bool FEAT>
+__global__ void __launch_bounds__(TPR_THREADS, 1) knn_tpr_kernel(const KnnParams p) {
+  // one row per thread.  The loops over the thread's rows are kept: written as scalar code the kernel compiles to
+  // different SASS (one to two more registers), so the row index r below is always 0.
+  constexpr int R = 1;
   constexpr int MODE = MODE_EXPANSION_NEG;
-  constexpr int THREADS = tpr_threads(R), WARPS = THREADS / 32;
+  constexpr int THREADS = TPR_THREADS, WARPS = THREADS / 32;
   extern __shared__ __align__(128) unsigned char smem[];
   const int N = p.N, k = KT ? KT : p.k;
   const int npad = tpr_npad(N), ntile = tpr_ntile(N);
@@ -96,9 +80,9 @@ __global__ void __launch_bounds__(tpr_threads(R), 1) knn_tpr_kernel(const KnnPar
 
   unsigned char* tail = smem + tpr_slots(N) * tpr_cloud_bytes(N);
   unsigned short* list = reinterpret_cast<unsigned short*>(tail) + tid;           // [R][TPR_CAP + 1][THREADS]
-  float* gmax = reinterpret_cast<float*>(tail + tpr_list_bytes(R)) + tid;         // [R][TPR_G][THREADS]
-  unsigned long long* cbuf = reinterpret_cast<unsigned long long*>(tail + tpr_list_bytes(R) + tpr_gmax_bytes(R)) + warp * 64;
-  int* wmax = reinterpret_cast<int*>(tail + tpr_list_bytes(R) + tpr_gmax_bytes(R) + (size_t)WARPS * 64 * 8);   // [2]
+  float* gmax = reinterpret_cast<float*>(tail + TPR_LIST_BYTES) + tid;         // [R][TPR_G][THREADS]
+  unsigned long long* cbuf = reinterpret_cast<unsigned long long*>(tail + TPR_LIST_BYTES + TPR_GMAX_BYTES) + warp * 64;
+  int* wmax = reinterpret_cast<int*>(tail + TPR_LIST_BYTES + TPR_GMAX_BYTES + (size_t)WARPS * 64 * 8);   // [2]
   constexpr int LIST_ROW = (TPR_CAP + 1) * THREADS;     // list entries per row index r
   constexpr int GMAX_ROW = TPR_G * THREADS;
 
@@ -157,10 +141,6 @@ __global__ void __launch_bounds__(tpr_threads(R), 1) knn_tpr_kernel(const KnnPar
       for (int r = 0; r < R; ++r) q[r] = packed[m0 + r * 32 + lane];
       unsigned slow_mask = p.force_slow ? (1u << R) - 1u : 0u;    // bit r: row r of this thread takes the exactness net
 
-#if L3D_TPR_STOP == 1
-      if (q[0].x == 12345.f) reinterpret_cast<long long*>(p.out_idx)[row0 * k] = 1;
-      continue;
-#endif
       if (!p.force_slow) {
         unsigned long long qx2[R], qy2[R], qz2[R];
 #pragma unroll
@@ -236,11 +216,6 @@ __global__ void __launch_bounds__(tpr_threads(R), 1) knn_tpr_kernel(const KnnPar
             for (int r = 0; r < R; ++r) gmax[r * GMAX_ROW + g * THREADS] = mx[r];
           }
         }
-#if L3D_TPR_STOP == 2
-        { float acc = 0.f;
-          for (int i = 0; i < R * TPR_G; ++i) acc += gmax[i * THREADS];
-          reinterpret_cast<long long*>(p.out_idx)[row0 * k] = (long long)__float_as_int(acc); continue; }
-#endif
         // ---- threshold per row: k-th largest of the 64 group maxima ----------------------------------------
         float thr_r[R];
 #pragma unroll 1
@@ -251,11 +226,11 @@ __global__ void __launch_bounds__(tpr_threads(R), 1) knn_tpr_kernel(const KnnPar
             const float* gm = gmax + r * GMAX_ROW;
 #pragma unroll
             for (int i = 0; i < 32; ++i) { ga[i] = gm[i * THREADS]; gb[i] = gm[(32 + i) * THREADS]; }
-            reg_sort_desc<32>(ga);
-            reg_sort_desc<32>(gb);
+            reg_sort_desc<32>(ga, cex_f32);
+            reg_sort_desc<32>(gb, cex_f32);
 #pragma unroll
             for (int i = 0; i < 32; ++i) ga[i] = fmaxf(ga[i], gb[31 - i]);    // the 32 largest of the 64, bitonic
-            reg_merge_desc<32>(ga);
+            reg_merge_desc<32>(ga, cex_f32);
             if (KT) {
               t0 = ga[KT ? KT - 1 : 0];
             } else {
@@ -264,12 +239,11 @@ __global__ void __launch_bounds__(tpr_threads(R), 1) knn_tpr_kernel(const KnnPar
               for (int i = 1; i < TPR_MAX_K; ++i) t0 = (i == k - 1) ? ga[i] : t0;
             }
           }
-          const float qw = (R == 2 && r == 1) ? q[R - 1].w : q[0].w;
+          const float qw = q[r].w;
           // s-space threshold (knn.cu row_threshold, DEFER): keeps every s whose key can reach the k-th group
           // maximum's key kb, admits at most the few s within ~2 ulp below it
           const float kb = __fsub_rn(t0, qw);
           float thr = __fadd_rd(__fadd_rd(kb, qw), -__fmul_rn(fmaxf(fabsf(kb), 1e-30f), 1.1920929e-7f));
-#if L3D_TPR_FUSE_THR
           // Pass 2 evaluates d = 2 (q.c - thr/2) - |c|^2 in ONE fma chain (the first product becomes an fma with the
           // addend -thr/2), i.e. s - thr with different roundings: |d - (s - thr)| <= 7 eps (|q|^2 + 2 max|c|^2 + |thr|),
           // eps = 2^-24 (three fma roundings of magnitude <= |q||c| + |thr|/2 <= (|q|^2 + |c|^2 + |thr|)/2, doubled, on
@@ -280,20 +254,12 @@ __global__ void __launch_bounds__(tpr_threads(R), 1) knn_tpr_kernel(const KnnPar
             const float delta = __fmul_ru(1.2e-6f, __fadd_ru(__fadd_ru(qw, wm), fabsf(thr)));
             thr = __fadd_rd(thr, -delta);
           }
-#endif
-          if (R == 2 && r == 1) thr_r[R - 1] = thr; else thr_r[0] = thr;
+          thr_r[r] = thr;
         }
-#if L3D_TPR_STOP == 3
-        { reinterpret_cast<long long*>(p.out_idx)[row0 * k] = (long long)__float_as_int(thr_r[0] + thr_r[R - 1]); continue; }
-#endif
-        unsigned long long hv[R];     // fused: (-thr/2, -thr/2) added inside the chain; else (-thr, -thr) added after it
+        unsigned long long hv[R];     // (-thr/2, -thr/2), added inside the pass-2 fma chain
 #pragma unroll
         for (int r = 0; r < R; ++r) {
-#if L3D_TPR_FUSE_THR
           hv[r] = f2_pack(-0.5f * thr_r[r], -0.5f * thr_r[r]);
-#else
-          hv[r] = f2_pack(-thr_r[r], -thr_r[r]);
-#endif
         }
 
         // ---- pass 2: survivor mask per 32 candidates, set bits appended to the row's index list ----------
@@ -326,7 +292,6 @@ __global__ void __launch_bounds__(tpr_threads(R), 1) knn_tpr_kernel(const KnnPar
           }
           return n0 + (n1 << 8);
         };
-        constexpr bool FUSED = (L3D_TPR_FUSE_THR != 0);
         {
           uint32_t mk_prev[R];     // the mask of word w - 1 is unpacked while word w is evaluated (independent work)
 #pragma unroll
@@ -341,33 +306,23 @@ __global__ void __launch_bounds__(tpr_threads(R), 1) knn_tpr_kernel(const KnnPar
             uint32_t lo16[R], hi16[R];
 #pragma unroll
             for (int r = 0; r < R; ++r) {
-              eval8(ax, az, t, qx2[r], qy2[r], qz2[r], FUSED, hv[r]);
-              if (!FUSED) {
-#pragma unroll
-                for (int i = 0; i < 8; ++i) t[i] = f2_add(t[i], hv[r]);
-              }
+              eval8(ax, az, t, qx2[r], qy2[r], qz2[r], true, hv[r]);
               lo16[r] = signs8(t);
             }
             load8(min(2 * w + 2, noct - 1), ax, az);
 #pragma unroll
             for (int r = 0; r < R; ++r) {
-              eval8(bx, bz, t, qx2[r], qy2[r], qz2[r], FUSED, hv[r]);
-              if (!FUSED) {
-#pragma unroll
-                for (int i = 0; i < 8; ++i) t[i] = f2_add(t[i], hv[r]);
-              }
+              eval8(bx, bz, t, qx2[r], qy2[r], qz2[r], true, hv[r]);
               hi16[r] = signs8(t);
             }
             load8(min(2 * w + 3, noct - 1), bx, bz);
 #pragma unroll
             for (int r = 0; r < R; ++r) {
               const uint32_t lend = lbase[r] + TPR_CAP * THREADS * 2;
-#if L3D_TPR_EXTRACT
               // a word holds 0.7 survivors on average: three branch-free steps, then a rarely entered loop
               take_lowest(mk_prev[r], laddr[r], lend, (w - 1) * 32);
               take_lowest(mk_prev[r], laddr[r], lend, (w - 1) * 32);
               take_lowest(mk_prev[r], laddr[r], lend, (w - 1) * 32);
-#endif
               while (mk_prev[r]) take_lowest(mk_prev[r], laddr[r], lend, (w - 1) * 32);
               mk_prev[r] = ~(lo16[r] + (hi16[r] << 16));
             }
@@ -376,16 +331,12 @@ __global__ void __launch_bounds__(tpr_threads(R), 1) knn_tpr_kernel(const KnnPar
           for (int r = 0; r < R; ++r)
             while (mk_prev[r]) take_lowest(mk_prev[r], laddr[r], lbase[r] + TPR_CAP * THREADS * 2, (nwords - 1) * 32);
         }
-#if L3D_TPR_STOP == 4
-        { reinterpret_cast<long long*>(p.out_idx)[row0 * k] = (long long)(laddr[0] + laddr[R - 1]); continue; }
-#endif
 
         // ---- final, one row at a time: composites of the first 32 survivors, in-register sort, store ------------
 #pragma unroll 1
         for (int r = 0; r < R; ++r) {
-          const bool second = (R == 2 && r == 1);
-          const float4 qr = second ? q[R - 1] : q[0];
-          const int cnt = (int)(((second ? laddr[R - 1] : laddr[0]) - (second ? lbase[R - 1] : lbase[0])) / (THREADS * 2));
+          const float4 qr = q[r];
+          const int cnt = (int)((laddr[r] - lbase[r]) / (THREADS * 2));
           const bool slow = cnt >= TPR_CAP;     // the saturated address means "TPR_CAP or more": exactness net below
           if (slow) slow_mask |= 1u << r;
           const unsigned short* lr = list + r * LIST_ROW;
@@ -398,7 +349,7 @@ __global__ void __launch_bounds__(tpr_threads(R), 1) knn_tpr_kernel(const KnnPar
             const unsigned long long c = tpr_composite(knn_key<MODE>(qr, packed[j]), j);
             a[i] = ok ? c : 0ull;
           }
-          tpr_sort_desc<32>(a);
+          reg_sort_desc<32>(a, tpr_cex);
           if (__any_sync(L3D_FULL_MASK, cnt > 32)) {
             // survivors 32..63 of the rows that have them: sort, keep the better 32 of the union, clean up
             unsigned long long bq[32];
@@ -409,10 +360,10 @@ __global__ void __launch_bounds__(tpr_threads(R), 1) knn_tpr_kernel(const KnnPar
               const unsigned long long c = tpr_composite(knn_key<MODE>(qr, packed[j]), j);
               bq[i] = ok ? c : 0ull;
             }
-            tpr_sort_desc<32>(bq);
+            reg_sort_desc<32>(bq, tpr_cex);
 #pragma unroll
             for (int i = 0; i < 32; ++i) a[i] = (bq[31 - i] > a[i]) ? bq[31 - i] : a[i];
-            tpr_merge_desc<32>(a);
+            reg_merge_desc<32>(a, tpr_cex);
           }
           // the k best (rank order): 128-bit stores when the row is 16-byte aligned
           if (!slow) {
@@ -449,7 +400,7 @@ __global__ void __launch_bounds__(tpr_threads(R), 1) knn_tpr_kernel(const KnnPar
 #pragma unroll 1
       for (int r = 0; r < R; ++r) {
         unsigned todo = __ballot_sync(L3D_FULL_MASK, (slow_mask >> r) & 1u);
-        const float4 qr = (R == 2 && r == 1) ? q[R - 1] : q[0];
+        const float4 qr = q[r];
         while (todo) {
           const int from = __ffs(todo) - 1;
           todo &= todo - 1;
@@ -491,13 +442,6 @@ __global__ void __launch_bounds__(tpr_threads(R), 1) knn_tpr_kernel(const KnnPar
 // owns row 32 h + lane.  The halves meet in shared memory (group maxima, thresholds, two index sub-lists per row),
 // the phases are separated by a 64-thread named barrier.  Rows per SM, warps per SM and fma work are unchanged;
 // shared-memory operand traffic halves.
-#ifndef L3D_DUO_UNROLL_G
-#define L3D_DUO_UNROLL_G 1   // candidate groups per pass-1 loop trip
-#endif
-#ifndef L3D_DUO_UNROLL_W
-#define L3D_DUO_UNROLL_W 1   // mask words per pass-2 loop trip
-#endif
-constexpr int DUO_UNROLL_G = L3D_DUO_UNROLL_G, DUO_UNROLL_W = L3D_DUO_UNROLL_W;
 constexpr int DUO_THREADS = 256, DUO_PER_CTA = DUO_THREADS / 64;
 constexpr int DUO_LCAP = 32;                 // entries per (row, candidate half) sub-list that count as "not full"
 constexpr int DUO_LROWS = DUO_LCAP + 4;      // + the entries the three unclamped steps of a word may touch
@@ -610,7 +554,7 @@ __global__ void __launch_bounds__(DUO_THREADS, 1) knn_duo_kernel(const KnnParams
         for (int r = 0; r < 2; ++r) { qx2[r] = f2_pack(q[r].x, q[r].x); qy2[r] = f2_pack(q[r].y, q[r].y); qz2[r] = f2_pack(q[r].z, q[r].z); }
         const unsigned long long two2 = f2_pack(2.0f, 2.0f);
         // ---- pass 1: maxima of this warp's 32 candidate groups, two rows per thread --------------------------
-#pragma unroll DUO_UNROLL_G
+#pragma unroll 1   // one group per trip (2 per trip: profiles/r02/knn_tpr_variants.txt)
         for (int gi = 0; gi < TPR_G / 2; ++gi) {
           const int g = h * (TPR_G / 2) + gi;
           const ulonglong2* gxy = pxy + g * ppg;
@@ -637,11 +581,11 @@ __global__ void __launch_bounds__(DUO_THREADS, 1) knn_duo_kernel(const KnnParams
           float ga[32], gb[32];
 #pragma unroll
           for (int i = 0; i < 32; ++i) { ga[i] = gmax_d[i * 64 + rho]; gb[i] = gmax_d[(32 + i) * 64 + rho]; }
-          reg_sort_desc<32>(ga);
-          reg_sort_desc<32>(gb);
+          reg_sort_desc<32>(ga, cex_f32);
+          reg_sort_desc<32>(gb, cex_f32);
 #pragma unroll
           for (int i = 0; i < 32; ++i) ga[i] = fmaxf(ga[i], gb[31 - i]);
-          reg_merge_desc<32>(ga);
+          reg_merge_desc<32>(ga, cex_f32);
           if (KT) {
             t0 = ga[KT ? KT - 1 : 0];
           } else {
@@ -678,7 +622,7 @@ __global__ void __launch_bounds__(DUO_THREADS, 1) knn_duo_kernel(const KnnParams
             mk ^= low;
           };
           const int w_begin = h * (nwords / 2), w_end = w_begin + nwords / 2;
-#pragma unroll DUO_UNROLL_W
+#pragma unroll 1   // one mask word per trip (2 per trip: profiles/r02/knn_tpr_variants.txt)
           for (int w = w_begin; w < w_end; ++w) {
             uint32_t m16[2][2];
 #pragma unroll
@@ -748,7 +692,7 @@ __global__ void __launch_bounds__(DUO_THREADS, 1) knn_duo_kernel(const KnnParams
             const unsigned long long c = tpr_composite(knn_key<MODE>(qo, packed[j]), j);
             a[i] = ok ? c : 0ull;
           }
-          tpr_sort_desc<32>(a);
+          reg_sort_desc<32>(a, tpr_cex);
           if (__any_sync(L3D_FULL_MASK, cnt > 32)) {
             unsigned long long bq[32];
 #pragma unroll
@@ -758,10 +702,10 @@ __global__ void __launch_bounds__(DUO_THREADS, 1) knn_duo_kernel(const KnnParams
               const unsigned long long c = tpr_composite(knn_key<MODE>(qo, packed[j]), j);
               bq[i] = ok ? c : 0ull;
             }
-            tpr_sort_desc<32>(bq);
+            reg_sort_desc<32>(bq, tpr_cex);
 #pragma unroll
             for (int i = 0; i < 32; ++i) a[i] = (bq[31 - i] > a[i]) ? bq[31 - i] : a[i];
-            tpr_merge_desc<32>(a);
+            reg_merge_desc<32>(a, tpr_cex);
           }
           // ---- output: the warp's 32 rows are one contiguous block of 32 k indices.  Every thread drops its k
           // indices as uint16 into a shared-memory image of that block (the duo's group-maximum array is free by
@@ -838,17 +782,6 @@ __global__ void __launch_bounds__(DUO_THREADS, 1) knn_duo_kernel(const KnnParams
 static thread_local int g_knn_path = 0;   // 0 auto, 1 warp-per-row-pair kernel only, 2 thread-per-row whenever eligible
 int knn_path_flag() { return g_knn_path; }
 
-static int tpr_sm_count() {
-  static int n = 0;
-  if (n == 0) {
-    int dev = 0;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev);
-    if (n <= 0) n = 148;
-  }
-  return n;
-}
-
 // shapes the thread-per-row kernel takes at all (the launcher in knn.cu adds the "enough rows" rule)
 bool knn_tpr_eligible(const KnnParams& p) {
   if (p.N % 32 != 0 || p.N < TPR_MIN_N || p.N > TPR_MAX_N || p.k > TPR_MAX_K || p.k < 1) return false;
@@ -856,94 +789,40 @@ bool knn_tpr_eligible(const KnnParams& p) {
   if ((reinterpret_cast<uintptr_t>(p.cand) & 7u) != 0) return false;       // float2 staging loads
   if (p.idx64 == 1 && (reinterpret_cast<uintptr_t>(p.out_idx) & 15u) != 0) return false;
   if (p.feat_out && p.idx64 != 1) return false;
-  return tpr_smem_bytes(p.N, 1) <= KNN_SMEM_LIMIT;
+  return tpr_smem_bytes(p.N) <= KNN_SMEM_LIMIT;
 }
 
-template <int R, int PPG, int KT, bool FEAT>
-static int tpr_launch_t(const KnnParams& p, cudaStream_t stream) {
-  auto kern = knn_tpr_kernel<R, PPG, KT, FEAT>;
-  const size_t smem = tpr_smem_bytes(p.N, R);
+// One CTA per SM, every CTA resident at once; a unit is `unit_rows` consecutive rows of one cloud.
+template <auto Kern>
+static int tpr_launch_t(const KnnParams& p, cudaStream_t stream, int threads, int unit_rows, size_t smem) {
   int dev = 0;
   cudaGetDevice(&dev);
-  {
-    // per-(device, function) attribute shared by every host thread: raise it once to the architectural maximum
-    static std::mutex mu;
-    static uint64_t done_mask = 0;
-    std::lock_guard<std::mutex> lock(mu);
-    if (dev >= 64 || !(done_mask >> dev & 1)) {
-      cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)KNN_SMEM_LIMIT);
-      if (e != cudaSuccess) return (int)e;
-      if (dev < 64) done_mask |= (uint64_t)1 << dev;
-    }
-  }
-  const long units = (long)p.B * (p.N / (32 * R));
-  long grid = tpr_sm_count();                      // one CTA per SM, every CTA resident at once
+  const cudaError_t e = raise_smem_once<Kern>(dev, KNN_SMEM_LIMIT);
+  if (e != cudaSuccess) return (int)e;
+  const long units = (long)p.B * (p.N / unit_rows);
+  long grid = sm_count(dev);
   if (grid > units) grid = units;
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3((unsigned)grid); cfg.blockDim = dim3(tpr_threads(R));
-  cfg.dynamicSmemBytes = smem; cfg.stream = stream;
-  cudaLaunchAttribute at[1];
-  at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  at[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = at; cfg.numAttrs = 1;
-  cudaError_t le = cudaLaunchKernelEx(&cfg, kern, p);
-  if (le != cudaSuccess) return (int)le;
-  count_launch();
-  L3D_LAUNCH_CHECK();
-  return L3D_OK;
-}
-
-template <int PPG, int KT, bool FEAT>
-static int duo_launch_t(const KnnParams& p, cudaStream_t stream) {
-  auto kern = knn_duo_kernel<PPG, KT, FEAT>;
-  const size_t smem = duo_smem_bytes(p.N);
-  int dev = 0;
-  cudaGetDevice(&dev);
-  {
-    static std::mutex mu;
-    static uint64_t done_mask = 0;
-    std::lock_guard<std::mutex> lock(mu);
-    if (dev >= 64 || !(done_mask >> dev & 1)) {
-      cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)KNN_SMEM_LIMIT);
-      if (e != cudaSuccess) return (int)e;
-      if (dev < 64) done_mask |= (uint64_t)1 << dev;
-    }
-  }
-  const long units = (long)p.B * (p.N / 64);
-  long grid = tpr_sm_count();                      // one CTA per SM, every CTA resident at once
-  if (grid > units) grid = units;
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3((unsigned)grid); cfg.blockDim = dim3(DUO_THREADS);
-  cfg.dynamicSmemBytes = smem; cfg.stream = stream;
-  cudaLaunchAttribute at[1];
-  at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  at[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = at; cfg.numAttrs = 1;
-  cudaError_t le = cudaLaunchKernelEx(&cfg, kern, p);
-  if (le != cudaSuccess) return (int)le;
-  count_launch();
-  L3D_LAUNCH_CHECK();
-  return L3D_OK;
+  return knn_launch_pdl(Kern, grid, threads, smem, stream, p);
 }
 
 int knn_tpr_launch(const KnnParams& p, cudaStream_t stream) {
   const bool n1024 = tpr_npad(p.N) == 1024;
-#if L3D_TPR_DUO
   if (p.N % 64 == 0 && duo_smem_bytes(p.N) <= KNN_SMEM_LIMIT) {
+    const size_t smem = duo_smem_bytes(p.N);
     if (p.feat_out) {
-      if (n1024 && p.k == 20) return duo_launch_t<8, 20, true>(p, stream);
-      return duo_launch_t<0, 0, true>(p, stream);
+      if (n1024 && p.k == 20) return tpr_launch_t<knn_duo_kernel<8, 20, true>>(p, stream, DUO_THREADS, 64, smem);
+      return tpr_launch_t<knn_duo_kernel<0, 0, true>>(p, stream, DUO_THREADS, 64, smem);
     }
-    if (n1024 && p.k == 20) return duo_launch_t<8, 20, false>(p, stream);
-    return duo_launch_t<0, 0, false>(p, stream);
+    if (n1024 && p.k == 20) return tpr_launch_t<knn_duo_kernel<8, 20, false>>(p, stream, DUO_THREADS, 64, smem);
+    return tpr_launch_t<knn_duo_kernel<0, 0, false>>(p, stream, DUO_THREADS, 64, smem);
   }
-#endif
+  const size_t smem = tpr_smem_bytes(p.N);
   if (p.feat_out) {
-    if (n1024 && p.k == 20) return tpr_launch_t<1, 8, 20, true>(p, stream);
-    return tpr_launch_t<1, 0, 0, true>(p, stream);
+    if (n1024 && p.k == 20) return tpr_launch_t<knn_tpr_kernel<8, 20, true>>(p, stream, TPR_THREADS, 32, smem);
+    return tpr_launch_t<knn_tpr_kernel<0, 0, true>>(p, stream, TPR_THREADS, 32, smem);
   }
-  if (n1024 && p.k == 20) return tpr_launch_t<1, 8, 20, false>(p, stream);
-  return tpr_launch_t<1, 0, 0, false>(p, stream);
+  if (n1024 && p.k == 20) return tpr_launch_t<knn_tpr_kernel<8, 20, false>>(p, stream, TPR_THREADS, 32, smem);
+  return tpr_launch_t<knn_tpr_kernel<0, 0, false>>(p, stream, TPR_THREADS, 32, smem);
 }
 
 }  // namespace l3d

@@ -1,134 +1,64 @@
 // In-register sorting networks and the 62-bit (key, index) composites of the thread-per-row selections
-// (knn_tpr.cu: knn() on xyz clouds; knn_matrix.cu: the selection stage of l3d_knn_features).
+// (knn_tpr.cu: knn() on xyz clouds).
 #pragma once
 #include "common.cuh"
-
-#ifndef L3D_TPR_DSETP
-#define L3D_TPR_DSETP 1       // 1: final sort compares 62-bit composites as positive doubles (DSETP on the fp64 pipe)
-#endif
 
 namespace l3d {
 
 // ---- in-register sorting networks (every index is a compile-time constant after unrolling) ----------------
-// Sorting networks: Batcher's merge exchange (Knuth 5.2.2 M) — 191 exchanges for 32 keys against 240 for the
-// bitonic sorter; every index is a compile-time constant after unrolling, the larger key ends at the lower index.
-template <int N>
-__device__ __forceinline__ void reg_sort_desc(float (&a)[N]) {
+// cex(x, y) is the compare-exchange: the larger element ends in x.  cex_f32 for group maxima, tpr_cex for the
+// composites below.
+// Sorting network: Batcher's merge exchange (Knuth 5.2.2 M) — 191 exchanges for 32 keys against 240 for the
+// bitonic sorter; the larger key ends at the lower index.
+template <int N, typename T, typename Cex>
+__device__ __forceinline__ void reg_sort_desc(T (&a)[N], Cex cex) {
 #pragma unroll
   for (int p = N / 2; p >= 1; p >>= 1) {
 #pragma unroll
     for (int i = 0; i < N - p; ++i)
-      if ((i & p) == 0) { const float hi = fmaxf(a[i], a[i + p]), lo = fminf(a[i], a[i + p]); a[i] = hi; a[i + p] = lo; }
+      if ((i & p) == 0) cex(a[i], a[i + p]);
 #pragma unroll
     for (int q = N / 2; q > p; q >>= 1) {
       const int d = q - p;
 #pragma unroll
       for (int i = 0; i < N - d; ++i)
-        if ((i & p) == p) { const float hi = fmaxf(a[i], a[i + d]), lo = fminf(a[i], a[i + d]); a[i] = hi; a[i + d] = lo; }
+        if ((i & p) == p) cex(a[i], a[i + d]);
     }
   }
 }
-template <int N>
-__device__ __forceinline__ void reg_merge_desc(float (&a)[N]) {   // a is bitonic -> descending
+template <int N, typename T, typename Cex>
+__device__ __forceinline__ void reg_merge_desc(T (&a)[N], Cex cex) {   // a is bitonic -> descending
 #pragma unroll
   for (int j = N >> 1; j > 0; j >>= 1) {
 #pragma unroll
     for (int i = 0; i < N; ++i) {
       const int l = i ^ j;
-      if (l > i) {
-        const float hi = fmaxf(a[i], a[l]), lo = fminf(a[i], a[l]);
-        a[i] = hi;
-        a[l] = lo;
-      }
+      if (l > i) cex(a[i], a[l]);
     }
   }
 }
-__device__ __forceinline__ void cex_u64(unsigned long long& x, unsigned long long& y, bool up) {
-  // one 64-bit comparison (ISETP + ISETP.EX) and four SELs per exchange.  Written in PTX: from C++ nvcc recognises
-  // the pair as umin/umax and emits a second, mirrored comparison for the minimum.
-  unsigned long long hi, lo;
-  asm("{\n\t.reg .pred p;\n\tsetp.gt.u64 p, %2, %3;\n\tselp.b64 %0, %2, %3, p;\n\tselp.b64 %1, %3, %2, p;\n\t}"
-      : "=l"(hi), "=l"(lo) : "l"(x), "l"(y));
-  x = up ? hi : lo;   // `up` is a compile-time constant after unrolling
-  y = up ? lo : hi;
-}
-template <int N>
-__device__ __forceinline__ void reg_sort_desc(unsigned long long (&a)[N]) {
-#pragma unroll
-  for (int k = 2; k <= N; k <<= 1) {
-#pragma unroll
-    for (int j = k >> 1; j > 0; j >>= 1) {
-#pragma unroll
-      for (int i = 0; i < N; ++i) {
-        const int l = i ^ j;
-        if (l > i) cex_u64(a[i], a[l], ((i & k) == 0) || k == N);
-      }
-    }
-  }
-}
-template <int N>
-__device__ __forceinline__ void reg_merge_desc(unsigned long long (&a)[N]) {
-#pragma unroll
-  for (int j = N >> 1; j > 0; j >>= 1) {
-#pragma unroll
-    for (int i = 0; i < N; ++i) {
-      const int l = i ^ j;
-      if (l > i) cex_u64(a[i], a[l], true);
-    }
-  }
+__device__ __forceinline__ void cex_f32(float& x, float& y) {
+  const float hi = fmaxf(x, y), lo = fminf(x, y);
+  x = hi;
+  y = lo;
 }
 
 // ---- final sort of the composites ---------------------------------------------------------------------------
-// L3D_TPR_DSETP: the composite is 62 bits, (ordered key << 30) | (~index & 0x3fffffff), so as an IEEE double it is a
-// non-negative finite number (or zero / denormal) whose numeric order is its bit-pattern order: one DSETP on the
-// fp64 pipe replaces the ISETP + ISETP.EX pair on the (busier) ALU pipe.
-#if L3D_TPR_DSETP
+// The composite is 62 bits, (ordered key << 30) | (~index & 0x3fffffff), so as an IEEE double it is a non-negative
+// finite number (or zero / denormal) whose numeric order is its bit-pattern order: one DSETP on the fp64 pipe
+// replaces the ISETP + ISETP.EX pair of a 64-bit integer comparison on the (busier) ALU pipe.
 __device__ __forceinline__ unsigned long long tpr_composite(float key, uint32_t idx) {
   return ((unsigned long long)f32_order(key + 0.0f) << 30) | (unsigned long long)(~idx & 0x3fffffffu);
 }
 __device__ __forceinline__ uint32_t tpr_comp_index(unsigned long long c) { return ~(uint32_t)c & 0x3fffffffu; }
 __device__ __forceinline__ float tpr_comp_key(unsigned long long c) { return f32_unorder((uint32_t)(c >> 30)); }
-__device__ __forceinline__ void tpr_cex(unsigned long long& x, unsigned long long& y, bool up) {
+__device__ __forceinline__ void tpr_cex(unsigned long long& x, unsigned long long& y) {
   unsigned long long hi, lo;
   asm("{\n\t.reg .pred p;\n\t.reg .f64 a, b;\n\tmov.b64 a, %2;\n\tmov.b64 b, %3;\n\tsetp.gt.f64 p, a, b;\n\t"
       "selp.b64 %0, %2, %3, p;\n\tselp.b64 %1, %3, %2, p;\n\t}"
       : "=l"(hi), "=l"(lo) : "l"(x), "l"(y));
-  x = up ? hi : lo;
-  y = up ? lo : hi;
+  x = hi;
+  y = lo;
 }
-#else
-__device__ __forceinline__ unsigned long long tpr_composite(float key, uint32_t idx) { return pack_pair(key, idx); }
-__device__ __forceinline__ uint32_t tpr_comp_index(unsigned long long c) { return ~(uint32_t)c; }
-__device__ __forceinline__ float tpr_comp_key(unsigned long long c) { return f32_unorder((uint32_t)(c >> 32)); }
-__device__ __forceinline__ void tpr_cex(unsigned long long& x, unsigned long long& y, bool up) { cex_u64(x, y, up); }
-#endif
-template <int N>
-__device__ __forceinline__ void tpr_sort_desc(unsigned long long (&a)[N]) {   // merge exchange, as reg_sort_desc
-#pragma unroll
-  for (int p = N / 2; p >= 1; p >>= 1) {
-#pragma unroll
-    for (int i = 0; i < N - p; ++i)
-      if ((i & p) == 0) tpr_cex(a[i], a[i + p], true);
-#pragma unroll
-    for (int q = N / 2; q > p; q >>= 1) {
-      const int d = q - p;
-#pragma unroll
-      for (int i = 0; i < N - d; ++i)
-        if ((i & p) == p) tpr_cex(a[i], a[i + d], true);
-    }
-  }
-}
-template <int N>
-__device__ __forceinline__ void tpr_merge_desc(unsigned long long (&a)[N]) {
-#pragma unroll
-  for (int j = N >> 1; j > 0; j >>= 1) {
-#pragma unroll
-    for (int i = 0; i < N; ++i) {
-      const int l = i ^ j;
-      if (l > i) tpr_cex(a[i], a[l], true);
-    }
-  }
-}
-
 
 }  // namespace l3d

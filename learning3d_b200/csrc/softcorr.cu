@@ -663,20 +663,15 @@ static __global__ void softcorr_merge_kernel(const float* __restrict__ part, int
 template <int EPI>
 static int sc_launch(SoftCorrParams p, void* stream) {
   if (p.B > 65535) return L3D_ERR_UNSUPPORTED;
-  // the opt-in shared-memory size is a per-device function attribute: cache per (thread, device)
-  static thread_local int attr_dev = -1;
   const size_t smem_t = softcorr_smem_bytes<true>(), smem_g = softcorr_smem_bytes<false>();
   const size_t smem_p = softcorr_smem_bytes<true, 2>();
   int dev = 0;
   cudaGetDevice(&dev);
-  if (attr_dev != dev) {
-    cudaError_t e = cudaFuncSetAttribute(softcorr_kernel<true, EPI>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_t);
+  {
+    cudaError_t e = raise_smem_once<softcorr_kernel<true, EPI>>(dev, smem_t);
+    if (e == cudaSuccess) e = raise_smem_once<softcorr_kernel<false, EPI>>(dev, smem_g);
+    if (e == cudaSuccess) e = raise_smem_once<softcorr_kernel<true, EPI, 2>>(dev, smem_p);
     if (e != cudaSuccess) return (int)e;
-    e = cudaFuncSetAttribute(softcorr_kernel<false, EPI>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_g);
-    if (e != cudaSuccess) return (int)e;
-    e = cudaFuncSetAttribute(softcorr_kernel<true, EPI, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_p);
-    if (e != cudaSuccess) return (int)e;
-    attr_dev = dev;
   }
   p.c = (float)(1.4426950408889634 / sqrt((double)p.D));
   void* errp = nullptr;
@@ -706,13 +701,8 @@ static int sc_launch(SoftCorrParams p, void* stream) {
   const int bn = tma ? SoftCorrCfg<true>::BN : SoftCorrCfg<false>::BN;
   const int tiles = (p.Nt + bn - 1) / bn;
   const long units = pair ? (long)((p.Ns + 2 * SC_BM - 1) / (2 * SC_BM)) * p.B : (long)grid.x * p.B;
-  static thread_local int sm_dev = -1, sm_count = 148;
-  if (sm_dev != dev) {
-    int n = 0;
-    if (cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev) == cudaSuccess && n > 0) sm_count = n;
-    sm_dev = dev;
-  }
-  const long slots = pair ? sm_count / 2 : sm_count;   // 1 CTA per SM; a pair needs both SMs of a TPC
+  const int sms = sm_count(dev);
+  const long slots = pair ? sms / 2 : sms;             // 1 CTA per SM; a pair needs both SMs of a TPC
   int jsplit = 1;
   if (EPI != EPI_STATS && EPI != EPI_DS && !(EPI == EPI_PROBS_T && p.probs_unnormalized) && g_softcorr_split >= 0 &&
       tiles > 1 && units * 2 <= slots) {

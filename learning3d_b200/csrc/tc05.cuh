@@ -163,10 +163,6 @@ __device__ __forceinline__ void tma_load_4d(uint32_t smem_dst, const CUtensorMap
 
 // L2 prefetch of one box (no shared memory, no barrier): hides HBM latency for tiles further ahead than the
 // shared-memory ring can hold (SASS: UTMAPF.L2)
-__device__ __forceinline__ void tma_prefetch_3d(const CUtensorMap* tmap, int c0, int c1, int c2) {
-  asm volatile("cp.async.bulk.prefetch.tensor.3d.L2.global.tile [%0, {%1, %2, %3}];" ::"l"(tmap), "r"(c0), "r"(c1), "r"(c2)
-               : "memory");
-}
 
 // Shared-memory matrix descriptors (cute::UMMA::SmemDescriptor, sm_100 "version 1"), SWIZZLE_128B.
 //   K-major  (generic path): rows of 32 fp32 (128 B), 8-row groups 1024 B apart (SBO).

@@ -1,5 +1,5 @@
-"""CPU check of the in-register sorting network of learning3d_b200/csrc/reg_sort.cuh (reg_sort_desc / tpr_sort_desc):
-the same loop nest restated in Python must be a sorting network (0/1 principle) with Batcher's merge-exchange size.
+"""CPU check of the in-register sorting network of learning3d_b200/csrc/reg_sort.cuh (reg_sort_desc, with either
+compare-exchange, cex_f32 or tpr_cex): the same loop nest restated in Python must be a sorting network (0/1 principle) with Batcher's merge-exchange size.
 The GPU suites only see its results; this pins the loop structure itself."""
 import itertools
 import random
